@@ -2,6 +2,7 @@
 """bench.py — the driver's measurement contract for the EasyLP B200 solve path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload pdlp|batch|transport|mcnf]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -38,6 +39,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it measures (which may be read-only)
 
 from oracle import gen  # noqa: E402  (seeded input generators; not a solve path)
 from easylp_b200.partition import lp_ranges, row_block  # noqa: E402
@@ -467,6 +469,7 @@ def bench_pdlp(args, dist, L, p, workload_name):
                                    "csr_gbs": (12 * nnzl + 4 * (ml + 1) + 8 * n + 8 * ml) / (ms_csr * 1e-3) / 1e9,
                                    "csc_gbs": (12 * nnzl + 4 * (n + 1) + 8 * ml + 8 * n) / (ms_csc * 1e-3) / 1e9}},
         "clocks": clocks,
+        "_outputs": {"x": x, "y": y, "objective": np.array([obj])},
     }
     if N > 1:
         L.comm_destroy()
@@ -535,6 +538,7 @@ def bench_batch(args, dist, L, d):
                      "ms_per_launch": ms,
                      "note": "HBM fraction is the mandated figure; shared-memory bandwidth and instruction issue of the pivot chain bound this kernel (ncu: LSU wavefronts 76 %, issue 56 %)"},
         "clocks": clocks,
+        "_outputs": {"status": status, "objective": obj, "x": x},
     }
 
 
@@ -634,6 +638,23 @@ def bench_lowering(args, L):
             "gpu_launches": low["gpu_launches"]}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy in float64, so that two builds can be compared output for output.  When the
+    arrays exceed DUMP_BYTES in all, each is cut to its share of the budget: a seeded sample of its flattened elements,
+    the same indices on every run with the same arguments."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.size * DUMP_BYTES // total
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def golden_objective(key):
     try:
@@ -719,7 +740,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--highs-lps", type=int, default=2000, help="LPs of config 3 given to the HiGHS stand-in")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary (batch) arm in the pdlp line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the primary arm's last timed step returned (x, y, objective of the PDLP solve; "
+                         "status, objective, x of the batch) as DIR/<name>.npy, float64, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         run_reference(args)
@@ -735,11 +761,13 @@ def main():
     if args.workload == "batch":
         d = gen.dense_batch(B=int(200_000 * args.scale), seed=0)
         res = bench_batch(args, dist, L, d)
+        outputs = res.pop("_outputs")
         if dist.rank == 0 and dist.world == 1 and not args.no_cpu_baseline:
             res["cpu_baseline"] = cpu_batch_baseline(d, min(d["B"], args.cpu_sample_lps), threads)
     else:
         p, name = make_problem(args)
         res = bench_pdlp(args, dist, L, p, name)
+        outputs = res.pop("_outputs")
         if not args.no_secondary:
             d = gen.dense_batch(B=int(200_000 * args.scale), seed=0)
             sec = bench_batch(args, dist, L, d)
@@ -776,6 +804,8 @@ def main():
                                                         gpu_c3_lps=res.get("batch", {}).get("e2e", {}).get("value"))
     if dist.rank == 0:
         print(json.dumps(res), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     dist.close()
     # the exit code carries parity: a wrong status / objective / residual at any N is a failed run, not a slow one
     bad = []
