@@ -12,11 +12,11 @@
 // relative KKT termination test.  The CPU restatement of this loop is oracle/pdlp_ref.py.
 //
 // Kernels per iteration (single GPU) — exactly two, both HBM-bound SpMVs with fused epilogues (spmv.cuh):
-//   K1  CSC (transposed) SpMV  g = A'y  + projection + reflection + Halpern combine  -> x, xbar
+//   K1  CSC (transposed) SpMV  g = A'y  + projection + reflection + Halpern combine  -> xbar (x is rebuilt from it)
 //   K2  CSR SpMV  A xbar       + dual prox + reflection + Halpern combine            -> y
 // Matrix stream, row pointers and the epilogue operands arrive in shared memory by TMA bulk copies;
 // the gathered vector (x: 8n bytes, y: 8m bytes) lives in the 126 MB L2.
-// Algorithmic bytes per iteration (DESIGN.md): 24 nnz + 4 (m+n+2) + 56 n + 40 m.
+// Algorithmic bytes per plain iteration (DESIGN.md §4.1): 24 nnz + 4 (m+n+2) + 8 (m+n) + 8 (4 + [l] + [u]) n + 33 m.
 //
 // Multi-GPU (SURVEY §8e): rank g owns a row block of A (for K2, its slice of y) AND a column block of A over all
 // rows (for K1, its slice of x).  Nothing is replicated; per iteration the x-bar blocks and the y blocks are
@@ -47,7 +47,7 @@ constexpr int SPMV_THREADS = 256;             // block size of the setup-only he
 // matrix stream, preload() picks this row's operands out of the stage, apply() runs after the row sum ------
 struct NoRoute {};
 struct StoreEpi {
-    static constexpr int NIN = 0;
+    static constexpr int NIN = 0, NINB = 0;
     static constexpr bool SCATTER = false;
     static constexpr bool DIST = false;
     double* scat = nullptr;
@@ -55,6 +55,7 @@ struct StoreEpi {
     using Route = NoRoute;
     struct Pre {};
     __device__ __forceinline__ const double* in(int) const { return nullptr; }
+    __device__ __forceinline__ const int8_t* in_b(int) const { return nullptr; }
     __device__ __forceinline__ Pre preload(const double*, int, int) const { return Pre{}; }
     __device__ __forceinline__ Pre preload_global(int) const { return Pre{}; }
     __device__ __forceinline__ double apply(int r, double s, const Pre&, const L2Hints&) const { out[r] = s; return 0.0; }
@@ -268,11 +269,31 @@ __device__ __forceinline__ void ghost_push_role(const GhostOut& go, int pw, int 
     }
 }
 
+// Halpern weight after k iterations of the epoch, and the iterate it forms: w xb + (1 - w) x0.  One rounding for every
+// place that forms x (the plain primal epilogue, its rebuild of x from the carried x-bar, k_halpern_finish): the rebuilt
+// x must be the stored one bit for bit.
+__host__ __device__ __forceinline__ double halpern_w(int k) { const double kd = (double)k; return (kd + 1.0) / (kd + 2.0); }
+__device__ __forceinline__ double halpern_x(double w, double xb, double x0) {
+    return __fma_rn(xb, w, __dmul_rn(__dadd_rn(1.0, -w), x0));
+}
+
+// bound kinds of the columns (after scaling), as template argument of the plain primal epilogue: a bound that is the
+// same constant in every column is not streamed
+constexpr int BND_L0 = 1;        // every l is +0.0 (bitwise: -0.0 keeps the stream)
+constexpr int BND_UINF = 2;      // every u is +inf
+
 // primal half of T(z) + reflection + Halpern combine.  g = (A'y)_j
 // GHOST (multi-GPU plain iterations): gathers y from this rank's ghost vector and publishes x-bar into the peers'.
-template <bool CHECK, bool GHOST = false>
+// Plain single-GPU iterations (CARRY) carry x-bar instead of x: x = halpern_x(w_prev, x-bar, x0) is rebuilt from the staged
+// operands, x-bar is overwritten in place (the dual kernel that gathers it has finished), and x itself is only stored
+// when `store_x` is set — by the last iteration of a chunk, for the check kernels that read it.  `from_x`: operand 0 is
+// x itself (x-bar does not belong to x, e.g. right after a restart).
+template <bool CHECK, bool GHOST = false, int BND = 0>
 struct PrimalEpi {
-    static constexpr int NIN = CHECK ? 4 : 5;
+    static constexpr bool CARRY = !CHECK && !GHOST;
+    static_assert(BND == 0 || CARRY, "constant bounds are a plain single-GPU specialisation");
+    static constexpr bool HAS_L = !(BND & BND_L0), HAS_U = !(BND & BND_UINF);
+    static constexpr int NIN = (CHECK ? 4 : 5) - !HAS_L - !HAS_U, NINB = 0;
     static constexpr bool SCATTER = false;
     static constexpr bool DIST = GHOST;
     double* scat;
@@ -287,34 +308,46 @@ struct PrimalEpi {
     int it;
     GhostIn gin;        // y ghost (consumed)
     GhostOut gout;      // x-bar ghosts (produced)
+    int from_x = 1, store_x = 1;      // CARRY only (see above)
     using Route = GhostRoute;
     struct Pre { double x, c, l, u, x0; };
+    __device__ __forceinline__ bool reads_xbar() const { return CARRY && !from_x; }
+    // operands: x (x-bar when carried), c, l, u, x0 — without the bounds BND makes constants, without x0 in a check
     __device__ __forceinline__ const double* in(int i) const {
-        return i == 0 ? x : i == 1 ? c : i == 2 ? l : i == 3 ? u : x0;
+        if (i == 0) return reads_xbar() ? xbar : x;
+        if (i == 1) return c;
+        if (HAS_L && i == 2) return l;
+        if (HAS_U && i == 2 + HAS_L) return u;
+        return x0;
     }
+    __device__ __forceinline__ const int8_t* in_b(int) const { return nullptr; }
     __device__ __forceinline__ Pre preload(const double* s, int rt, int g) const {
         Pre p;
-        p.x = s[g]; p.c = s[rt + g]; p.l = s[2 * rt + g]; p.u = s[3 * rt + g];
-        p.x0 = CHECK ? 0.0 : s[(CHECK ? 0 : 4) * rt + g];
+        p.x = s[g]; p.c = s[rt + g];
+        p.l = HAS_L ? s[2 * rt + g] : 0.0;
+        p.u = HAS_U ? s[(2 + HAS_L) * rt + g] : INFINITY;
+        p.x0 = CHECK ? 0.0 : s[(NIN - 1) * rt + g];
         return p;
     }
     __device__ __forceinline__ Pre preload_global(int j) const {
         Pre p;
-        p.x = x[j]; p.c = c[j]; p.l = l[j]; p.u = u[j];
+        p.x = reads_xbar() ? xbar[j] : x[j]; p.c = c[j];
+        p.l = HAS_L ? l[j] : 0.0;
+        p.u = HAS_U ? u[j] : INFINITY;
         p.x0 = CHECK ? 0.0 : x0[j];
         return p;
     }
     __device__ __forceinline__ double apply(int j, double g, const Pre& p, const L2Hints& h) const {
         const double tau = P->tau;
-        const double xpj = fmin(fmax(p.x - tau * (p.c - g), p.l), p.u);
-        const double xb = 2.0 * xpj - p.x;
+        // the previous iteration formed x with the weight of k - 1
+        const double xk = reads_xbar() ? halpern_x(halpern_w(P->k_base + it - 1), p.x, p.x0) : p.x;
+        const double xpj = fmin(fmax(xk - tau * (p.c - g), p.l), p.u);
+        const double xb = 2.0 * xpj - xk;
         if (!GHOST) st_out(xbar + j, xb, h, true);
         if (CHECK) {
             xp[j] = xpj;
-        } else {
-            const double k = (double)(P->k_base + it);
-            const double w = (k + 1.0) / (k + 2.0);
-            st_out(x + j, w * xb + (1.0 - w) * p.x0, h, false);
+        } else if (!CARRY || store_x) {
+            st_out(x + j, halpern_x(halpern_w(P->k_base + it), xb, p.x0), h, false);
         }
         return GHOST ? xb : 0.0;
     }
@@ -334,9 +367,12 @@ struct PrimalEpi {
 // dual half.  ax = (A xbar)_i.  SCAT: the kernel then adds val[k] * y_new_i into scat[idx[k]] over the entries of row i,
 // i.e. it leaves g = A'y_new behind for the next (gather-free) primal update.
 // GHOST (multi-GPU plain iterations): gathers x-bar from this rank's ghost vector and publishes y into the peers'.
-template <bool CHECK, bool SCAT = false, bool GHOST = false>
+// RHS (plain single-GPU iterations): the row bounds are rebuilt from the scaled right-hand side and the sense byte,
+// lc = (LE ? -inf : rhs), uc = (GE ? +inf : rhs) — 9 bytes per row instead of 16; only where that gives lc / uc exactly.
+template <bool CHECK, bool SCAT = false, bool GHOST = false, bool RHS = false>
 struct DualEpi {
-    static constexpr int NIN = CHECK ? 3 : 4;
+    static_assert(!RHS || (!CHECK && !SCAT && !GHOST), "the rhs + sense stream is a plain single-GPU specialisation");
+    static constexpr int NIN = CHECK || RHS ? 3 : 4, NINB = RHS ? 1 : 0;
     static constexpr bool SCATTER = SCAT;
     static constexpr bool DIST = GHOST;
     double* scat;
@@ -350,18 +386,32 @@ struct DualEpi {
     int it;
     GhostIn gin;        // x-bar ghost (consumed)
     GhostOut gout;      // y ghosts (produced)
+    const double* __restrict__ rhs = nullptr;     // RHS only: scaled right-hand side and sense of every row
+    const int8_t* __restrict__ sense = nullptr;
     using Route = GhostRoute;
     struct Pre { double y, lc, uc, y0; };
-    __device__ __forceinline__ const double* in(int i) const { return i == 0 ? y : i == 1 ? lc : i == 2 ? uc : y0; }
+    __device__ __forceinline__ const double* in(int i) const {
+        if (RHS) return i == 0 ? y : i == 1 ? rhs : y0;
+        return i == 0 ? y : i == 1 ? lc : i == 2 ? uc : y0;
+    }
+    __device__ __forceinline__ const int8_t* in_b(int) const { return sense; }
+    static __device__ __forceinline__ void bounds_of(int sn, double r, Pre& p) {
+        p.lc = sn == ELP_LE ? -INFINITY : r;
+        p.uc = sn == ELP_GE ? INFINITY : r;
+    }
     __device__ __forceinline__ Pre preload(const double* s, int rt, int g) const {
         Pre p;
-        p.y = s[g]; p.lc = s[rt + g]; p.uc = s[2 * rt + g];
-        p.y0 = CHECK ? 0.0 : s[(CHECK ? 0 : 3) * rt + g];
+        p.y = s[g];
+        if (RHS) bounds_of(reinterpret_cast<const int8_t*>(s + NIN * rt)[g], s[rt + g], p);
+        else { p.lc = s[rt + g]; p.uc = s[2 * rt + g]; }
+        p.y0 = CHECK ? 0.0 : s[(NIN - 1) * rt + g];
         return p;
     }
     __device__ __forceinline__ Pre preload_global(int i) const {
         Pre p;
-        p.y = y[i]; p.lc = lc[i]; p.uc = uc[i];
+        p.y = y[i];
+        if (RHS) bounds_of(sense[i], rhs[i], p);
+        else { p.lc = lc[i]; p.uc = uc[i]; }
         p.y0 = CHECK ? 0.0 : y0[i];
         return p;
     }
@@ -507,6 +557,27 @@ __global__ void k_row_bounds(int m, const int8_t* __restrict__ sense, const doub
     lc[i] = (s == ELP_LE) ? -INFINITY : r;
     uc[i] = (s == ELP_GE) ? INFINITY : r;
 }
+// setup: bit 0 some l is not +0.0, bit 1 some u is not +inf, bit 2 some row whose lc / uc are not what rhs and sense
+// rebuild (DualEpi<RHS>), compared bit for bit
+__global__ void k_bound_kinds(int n, const double* __restrict__ l, const double* __restrict__ u, int m,
+                              const int8_t* __restrict__ sense, const double* __restrict__ rhs, const double* __restrict__ lc,
+                              const double* __restrict__ uc, unsigned int* __restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned int f = 0;
+    if (i < n) {
+        if (__double_as_longlong(l[i]) != 0) f |= 1u;
+        if (__double_as_longlong(u[i]) != __double_as_longlong(INFINITY)) f |= 2u;
+    }
+    if (i < m) {
+        const int s = sense[i];
+        const double r = rhs[i];
+        if (__double_as_longlong(s == ELP_LE ? -INFINITY : r) != __double_as_longlong(lc[i]) ||
+            __double_as_longlong(s == ELP_GE ? INFINITY : r) != __double_as_longlong(uc[i]))
+            f |= 4u;
+    }
+    f = __reduce_or_sync(0xffffffffu, f);
+    if ((threadIdx.x & 31) == 0 && f) atomicOr(out, f);
+}
 __global__ void k_init_x(int n, double* __restrict__ x, const double* __restrict__ l, const double* __restrict__ u) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j < n) x[j] = fmin(fmax(0.0, l[j]), u[j]);
@@ -523,7 +594,7 @@ __global__ void k_halpern_finish(int n, double* __restrict__ x, const double* __
                                  const double* __restrict__ x0, int m, double* __restrict__ y,
                                  const double* __restrict__ yp, const double* __restrict__ y0, double w) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) x[i] = w * xbar[i] + (1.0 - w) * x0[i];
+    if (i < n) x[i] = halpern_x(w, xbar[i], x0[i]);
     if (i < m) y[i] = w * (2.0 * yp[i] - y[i]) + (1.0 - w) * y0[i];
 }
 // restart: iterate and anchor both jump to the candidate T(z)
@@ -880,6 +951,10 @@ struct Pdlp {
     // vectors (scaled); column-side ones have nl entries, row-side ones m
     DevBuf<double> c, l, u, dc, x, x0, xp, gcol;
     DevBuf<double> lc, uc, dr, y0, yp, axbar, axp;
+    DevBuf<double> rs;           // scaled right-hand side: lc = (LE ? -inf : rs), uc = (GE ? +inf : rs)
+    DevBuf<int8_t> rsense;       // row senses, padded to 16-byte copies
+    int pbnd = 0;                // plain iterations: bounds that are constants (BND_L0 | BND_UINF), single GPU
+    bool drhs = false;           // plain iterations: the dual epilogue streams rs + rsense instead of lc + uc
     DevBuf<double> xbar_full, y_full, xaux_full, yaux_full;   // [N*nb], [N*mb]: gathered vectors + scratch
     // peer-store exchange (N > 1, CUDA IPC): every rank's xbar_full / y_full / flag rows mapped here
     bool scatter = false;        // plain iterations: g = A'y accumulated by the dual kernel's scatter (single GPU only)
@@ -1322,8 +1397,8 @@ struct Pdlp {
             const size_t nbg = (size_t)((ceil_div(n, N) + 3) & ~3), sxg = (size_t)N * nbg;
             const size_t mbg = (size_t)m + m / 8 + 64, syg = (size_t)N * mbg;          // padded rows per rank: a guess
             const size_t nnzc_g = (size_t)(1.3 * (double)nnz) + (1u << 20);
-            arena.reserve((size_t)16 * nnz + (size_t)16 * nnzc_g + (size_t)8 * (10 * nbg + 9 * (size_t)m) + (size_t)16 * (sxg + syg) +
-                          (size_t)2 * (nbg + m) + (size_t)4 * syg + (4u << 20));
+            arena.reserve((size_t)16 * nnz + (size_t)16 * nnzc_g + (size_t)8 * (10 * nbg + 10 * (size_t)m) + (size_t)16 * (sxg + syg) +
+                          (size_t)3 * (nbg + m) + (size_t)4 * syg + (4u << 20));
             scratch.reserve((size_t)52 * nnz + (size_t)12 * nnzc_g + (size_t)16 * ((size_t)n + m) + (size_t)N * (sxg + syg) +
                             (size_t)8 * std::max(sxg, syg) + (size_t)16 * sxg + (16u << 20));
         }
@@ -1351,10 +1426,12 @@ struct Pdlp {
         // epilogue operands are staged by 16-byte-granular bulk copies: SPMV_VPAD doubles of slack each
         const size_t np = (size_t)std::max(nl, 1) + SPMV_VPAD, mp = (size_t)std::max(m, 1) + SPMV_VPAD;
         c.alloc(np); l.alloc(np); u.alloc(np); dc.alloc(np); x.alloc(np); x0.alloc(np); xp.alloc(np); gcol.alloc(np);
-        lc.alloc(mp); uc.alloc(mp); dr.alloc(mp); y0.alloc(mp); yp.alloc(mp); axbar.alloc(mp); axp.alloc(mp);
+        lc.alloc(mp); uc.alloc(mp); dr.alloc(mp); y0.alloc(mp); yp.alloc(mp); axbar.alloc(mp); axp.alloc(mp); rs.alloc(mp);
+        rsense.alloc((size_t)((std::max(m, 1) + 15) & ~15));
+        rsense.zero(st);
         xbar_full.alloc((size_t)N * nb + SPMV_VPAD); xaux_full.alloc((size_t)N * nb + SPMV_VPAD);
         y_full.alloc((size_t)N * mb + SPMV_VPAD); yaux_full.alloc((size_t)N * mb + SPMV_VPAD);
-        for (DevBuf<double>* b : {&c, &l, &u, &dc, &x, &x0, &xp, &gcol, &lc, &uc, &dr, &y0, &yp, &axbar, &axp, &xbar_full,
+        for (DevBuf<double>* b : {&c, &l, &u, &dc, &x, &x0, &xp, &gcol, &lc, &uc, &dr, &y0, &yp, &axbar, &axp, &rs, &xbar_full,
                                   &xaux_full, &y_full, &yaux_full})
             b->zero(st);
 
@@ -1374,15 +1451,9 @@ struct Pdlp {
         }
         c.upload(c_h + n0, nl, st); l.upload(lb + n0, nl, st); u.upload(ub + n0, nl, st);
         h2d += (int64_t)nl * 24;
-        {
-            ArenaScope tmp(scratch.base ? &scratch : g_arena);
-            DevBuf<int8_t> sense_d(std::max(m, 1));
-            DevBuf<double> rhs_d(std::max(m, 1));
-            sense_d.upload(sense, m, st); rhs_d.upload(rhs, m, st);
-            h2d += (int64_t)m * 9;
-            if (m > 0) ELP_LAUNCH(k_row_bounds, grid1(m), 256, 0, st, m, sense_d.p, rhs_d.p, lc.p, uc.p);
-            ELP_CUDA(cudaStreamSynchronize(st));
-        }
+        rsense.upload(sense, m, st); rs.upload(rhs, m, st);
+        h2d += (int64_t)m * 9;
+        if (m > 0) ELP_LAUNCH(k_row_bounds, grid1(m), 256, 0, st, m, rsense.p, rs.p, lc.p, uc.p);
         if (maximize && nl > 0) ELP_LAUNCH(k_scale_scalar, grid1(nl), 256, 0, st, nl, c.p, -1.0);
 
         mark("upload");
@@ -1431,6 +1502,7 @@ struct Pdlp {
         fetch_scalars(h);
         const double ncn = std::sqrt(h[0]);
         w_init = (nbn > 1e-10 && ncn > 1e-10) ? ncn / nbn : 1.0;
+        choose_streams();
         setup_ghost_exchange();
         reset();
         mark("reset");
@@ -1565,7 +1637,29 @@ struct Pdlp {
         if (m > 0) {
             ELP_LAUNCH(k_mul, grid1(m), 256, 0, st, m, lc.p, dr.p);
             ELP_LAUNCH(k_mul, grid1(m), 256, 0, st, m, uc.p, dr.p);
+            ELP_LAUNCH(k_mul, grid1(m), 256, 0, st, m, rs.p, dr.p);
         }
+    }
+
+    // Single GPU: which operand streams of the plain iterations the scaled problem can do without (pbnd, drhs)
+    void choose_streams() {
+        pbnd = 0; drhs = false;
+        if (N > 1) return;
+        unsigned int hf = 0;
+        {
+            ArenaScope tmp(scratch.base ? &scratch : nullptr);
+            DevBuf<unsigned int> f(1);
+            f.zero(st);
+            const int span = std::max(nl, m);
+            if (span > 0) ELP_LAUNCH(k_bound_kinds, grid1(span), 256, 0, st, nl, l.p, u.p, m, rsense.p, rs.p, lc.p, uc.p, f.p);
+            f.download(&hf, 1, st);
+            ELP_CUDA(cudaStreamSynchronize(st));
+        }
+        pbnd = ((hf & 1u) ? 0 : BND_L0) | ((hf & 2u) ? 0 : BND_UINF);
+        drhs = !(hf & 4u) && (plan_r.rowwarp || plan_r.L <= 2);     // a sense byte per row needs tiles of >= 16 rows
+        if (opt.verbose > 0 || env_int("ELP_PDLP_DEBUG", 0))
+            fprintf(stderr, "[pdlp] plain iterations stream %s%s and %s\n", (pbnd & BND_L0) ? "" : "l ",
+                    (pbnd & BND_UINF) ? "" : "u", drhs ? "rhs + sense" : "lc + uc");
     }
 
     void estimate_sigma_max() {
@@ -1638,8 +1732,16 @@ struct Pdlp {
     void signal_only(const GhostIn& gi, int plus) {
         ELP_LAUNCH(k_ghost_signal_only, 1, 32, 0, st, gi, params.p, plus);
     }
+    template <int BND>
+    void launch_primal_plain(int it, int from_x, int store_x) {
+        PrimalEpi<false, false, BND> epi{nullptr, c.p, l.p, u.p, x0.p, x.p, xbar(), xp.p, params.p, it, GhostIn{}, GhostOut{},
+                                         from_x, store_x};
+        launch_spmv(plan_c, nl, csc_ptr.p, csc_idx.p, csc_val.p, y_full.p, epi, st);
+    }
+    // plain iterations: store_x on the last one before a check or the end of run() (see PrimalEpi), from_x when x-bar
+    // does not belong to x
     template <bool CHECK>
-    void primal_step(int it) {
+    void primal_step(int it, bool store_x = true, bool from_x = false) {
         if (!CHECK && scatter) {            // g = A'y is already in gcol (left there by the dual kernel's scatter)
             const int grid = std::max(1, std::min(ceil_div(nl / 2, 256), kNumSMs * 8));
             ELP_LAUNCH(k_primal_from_g, grid, 256, 0, st, nl, gcol.p, c.p, l.p, u.p, x0.p, x.p, xbar(), params.p, it);
@@ -1651,8 +1753,19 @@ struct Pdlp {
             else signal_only(yin, it);            // what K1's prologue would have said: my y of the previous epoch is out
             return;
         }
-        PrimalEpi<CHECK> epi{nullptr, c.p, l.p, u.p, x0.p, x.p, xbar(), xp.p, params.p, it, GhostIn{}, GhostOut{}};
-        launch_spmv(plan_c, nl, csc_ptr.p, csc_idx.p, csc_val.p, y_full.p, epi, st);
+        if constexpr (CHECK) {
+            PrimalEpi<true> epi{nullptr, c.p, l.p, u.p, x0.p, x.p, xbar(), xp.p, params.p, it, GhostIn{}, GhostOut{}};
+            launch_spmv(plan_c, nl, csc_ptr.p, csc_idx.p, csc_val.p, y_full.p, epi, st);
+        } else {
+            // N > 1 (all-gather exchange): x stays the stored iterate
+            const int fx = N > 1 || from_x, sx = N > 1 || store_x;
+            switch (pbnd) {
+                case 0: launch_primal_plain<0>(it, fx, sx); break;
+                case BND_L0: launch_primal_plain<BND_L0>(it, fx, sx); break;
+                case BND_UINF: launch_primal_plain<BND_UINF>(it, fx, sx); break;
+                default: launch_primal_plain<BND_L0 | BND_UINF>(it, fx, sx); break;
+            }
+        }
         gather_x(xbar_full.p);
     }
     template <bool CHECK>
@@ -1668,8 +1781,14 @@ struct Pdlp {
             else signal_only(xin, it + 1);        // what K2's prologue would have said: my x-bar of this epoch is out
             return;
         }
-        DualEpi<CHECK> epi{nullptr, lc.p, uc.p, y0.p, y(), yp.p, axbar.p, params.p, it, GhostIn{}, GhostOut{}};
-        launch_spmv(plan_r, m, csr_ptr.p, csr_idx.p, csr_val.p, xbar_full.p, epi, st);
+        if (!CHECK && drhs) {
+            DualEpi<false, false, false, true> epi{nullptr, lc.p, uc.p, y0.p, y(), yp.p, axbar.p, params.p, it, GhostIn{}, GhostOut{},
+                                                   rs.p, rsense.p};
+            launch_spmv(plan_r, m, csr_ptr.p, csr_idx.p, csr_val.p, xbar_full.p, epi, st);
+        } else {
+            DualEpi<CHECK> epi{nullptr, lc.p, uc.p, y0.p, y(), yp.p, axbar.p, params.p, it, GhostIn{}, GhostOut{}};
+            launch_spmv(plan_r, m, csr_ptr.p, csr_idx.p, csr_val.p, xbar_full.p, epi, st);
+        }
         if (!CHECK) gather_y(y_full.p);                      // a check iteration does not change y here
     }
     int kernels_per_iter() const { return ghost ? 2 : (m > 0 ? 1 : 0) + (nl > 0 ? 1 : 0); }
@@ -1684,7 +1803,7 @@ struct Pdlp {
                 const int64_t before = g_launches.load();
                 ELP_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
                 try {
-                    for (int i = 0; i < count; ++i) { primal_step<false>(i); dual_step<false>(i); }
+                    for (int i = 0; i < count; ++i) { primal_step<false>(i, i == count - 1); dual_step<false>(i); }
                 } catch (...) {
                     cudaStreamEndCapture(st, &g);
                     if (g) cudaGraphDestroy(g);
@@ -1699,7 +1818,7 @@ struct Pdlp {
             ELP_CUDA(cudaGraphLaunch(graph, st));
             g_launches.fetch_add((int64_t)count * kernels_per_iter());
         } else {
-            for (int i = 0; i < count; ++i) { primal_step<false>(i); dual_step<false>(i); }
+            for (int i = 0; i < count; ++i) { primal_step<false>(i, i == count - 1); dual_step<false>(i); }
         }
         k += count;
         total += count;
@@ -1798,7 +1917,7 @@ struct Pdlp {
             ELP_LAUNCH(k_restart, grid1(span), 256, 0, st, nl, x.p, x0.p, xp.p, m, y(), y0.p, yp.p);
             k = 0; ++restarts; need_fpe0 = true; fpe_prev = -1;
         } else {
-            const double wk = (k + 1.0) / (k + 2.0);
+            const double wk = halpern_w(k);
             ELP_LAUNCH(k_halpern_finish, grid1(span), 256, 0, st, nl, x.p, xbar(), x0.p, m, y(), yp.p, y0.p, wk);
             ++k;
         }
@@ -1928,11 +2047,12 @@ struct Pdlp {
         run(3 * std::max(2, opt.check_every), nullptr);
         std::vector<cudaEvent_t> ev(2 * (size_t)reps + 1);
         for (auto& e : ev) ELP_CUDA(cudaEventCreate(&e));
-        // real iterations, exchange included (multi-GPU: the peers run the same sequence)
-        for (int i = 0; i < 3; ++i) { primal_step<false>(i); dual_step<false>(i); }
+        // real iterations, exchange included (multi-GPU: the peers run the same sequence).  run() may have ended with a
+        // restart (x-bar stale): the first one reads x itself.
+        for (int i = 0; i < 3; ++i) { primal_step<false>(i, false, i == 0); dual_step<false>(i); }
         for (int i = 0; i < reps; ++i) {
             ELP_CUDA(cudaEventRecord(ev[2 * i], st));
-            primal_step<false>(3 + i);
+            primal_step<false>(3 + i, false);
             ELP_CUDA(cudaEventRecord(ev[2 * i + 1], st));
             dual_step<false>(3 + i);
         }

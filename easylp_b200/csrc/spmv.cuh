@@ -12,7 +12,7 @@
 //     warp-strided round-robin) and owns a private ring of NSTW stages in shared memory with one mbarrier
 //     each.  No CTA-wide or inter-warp synchronisation exists in the loop;
 //   * EVERYTHING that streams — the tile's slice of val/idx, its row pointers and the epilogue's operand
-//     vectors (x, c, l, u, x0 / y, lc, uc, y0) — is brought into the ring by 1-D TMA bulk copies
+//     vectors (x-bar, c, l, u, x0 / y, rhs, y0 and a sense byte per row) — is brought into the ring by 1-D TMA bulk copies
 //     (cp.async.bulk -> mbarrier complete_tx); lane i of the warp issues copy i, NSTW tiles ahead of the
 //     tile being consumed, so the HBM latency is covered by the ring and not by the warp's own loads;
 //   * the only loads the lanes issue to global memory are the gathers vec[idx[k]] (random 8-byte read-only
@@ -41,13 +41,14 @@ struct SpmvStageLayout {          // byte offsets inside one stage of one warp
     int cap;                      // entries per stage (multiple of 4)
     int off_idx, off_ptr, off_ops, off_route, bytes;
 };
-__host__ __device__ inline SpmvStageLayout spmv_stage_layout(int cap, int rw, int nin, bool route = false) {
+// nin operand vectors of doubles, then ninb of bytes (16-byte copies: only for tiles of a multiple of 16 rows)
+__host__ __device__ inline SpmvStageLayout spmv_stage_layout(int cap, int rw, int nin, bool route = false, int ninb = 0) {
     SpmvStageLayout s;
     s.cap = cap;
     s.off_idx = cap * 8;
     s.off_ptr = s.off_idx + cap * 4;
     s.off_ops = s.off_ptr + (rw + 4) * 4;
-    s.off_route = s.off_ops + nin * ((rw + 1) & ~1) * 8;
+    s.off_route = s.off_ops + nin * ((rw + 1) & ~1) * 8 + ninb * ((rw + 15) & ~15);
     s.off_route = (s.off_route + 15) & ~15;
     s.bytes = s.off_route + (route ? SPMV_ROUTE_WORDS * 4 : 0);
     s.bytes = (s.bytes + 15) & ~15;
@@ -64,11 +65,12 @@ spmv_warp_kernel(int nrows, int ntiles, int cap, const int* __restrict__ ptr, co
     // hold a stage a little longer)
     constexpr int G = 32 / L;                // lane groups per warp
     constexpr int RW = G * RPL;              // rows per warp tile: group g owns rows g, g + G, ...
-    constexpr int NIN = Epi::NIN;
+    constexpr int NIN = Epi::NIN, NINB = Epi::NINB;
+    static_assert(NINB == 0 || RW % 16 == 0, "byte operands are staged in 16-byte pieces: tiles of a multiple of 16 rows");
     constexpr int U = (L <= 2) ? 8 : 4;      // gathers in flight per lane
     constexpr int OPS = (RW + 1) & ~1;       // doubles per staged operand
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    const SpmvStageLayout lay = spmv_stage_layout(cap, RW, NIN, Epi::DIST);
+    const SpmvStageLayout lay = spmv_stage_layout(cap, RW, NIN, Epi::DIST, NINB);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     unsigned char* ring = smem_raw + (size_t)warp * NSTW * lay.bytes;
     uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)SPMV_WARPS * NSTW * lay.bytes) + warp * NSTW;
@@ -120,6 +122,7 @@ spmv_warp_kernel(int nrows, int ntiles, int cap, const int* __restrict__ ptr, co
         const int rows = min(RW, nrows - r0);
         const uint32_t ptr_bytes = (uint32_t)((rows + 1 + 3) & ~3) * 4u;
         const uint32_t op_bytes = (uint32_t)((rows + 1) & ~1) * 8u;
+        const uint32_t opb_bytes = (uint32_t)((rows + 15) & ~15);
         unsigned char* sb = ring + (size_t)stage * lay.bytes;
         // lane i issues copy i: 0 val, 1 idx, 2 row pointers, 3.. epilogue operands
         const void* src = nullptr;
@@ -130,7 +133,12 @@ spmv_warp_kernel(int nrows, int ntiles, int cap, const int* __restrict__ ptr, co
         else if (p_piece == 0) {
             if (lane == 2) { src = ptr + r0; dst = sb + lay.off_ptr; bytes = ptr_bytes; }
             else if (lane < 3 + NIN) { src = epi.in(lane - 3) + r0; dst = sb + lay.off_ops + (lane - 3) * OPS * 8; bytes = op_bytes; }
-            else if (lane == 3 + NIN) {
+            else if (lane < 3 + NIN + NINB) {
+                src = epi.in_b(lane - 3 - NIN) + r0;
+                dst = sb + lay.off_ops + NIN * OPS * 8 + (lane - 3 - NIN) * ((RW + 15) & ~15);
+                bytes = opb_bytes;
+            }
+            else if (lane == 3 + NIN + NINB) {
                 if constexpr (Epi::DIST) {                // multi-GPU: the tile's routing record travels with its operands
                     if (epi.route_table() != nullptr) {
                         src = epi.route_table() + (size_t)p_tile * SPMV_ROUTE_WORDS; dst = sb + lay.off_route; bytes = SPMV_ROUTE_WORDS * 4;
@@ -140,7 +148,7 @@ spmv_warp_kernel(int nrows, int ntiles, int cap, const int* __restrict__ ptr, co
         }
         if (lane == 0) {
             uint32_t tx = (uint32_t)pcnt * 12u;
-            if (p_piece == 0) tx += ptr_bytes + (uint32_t)NIN * op_bytes;
+            if (p_piece == 0) tx += ptr_bytes + (uint32_t)NIN * op_bytes + (uint32_t)NINB * opb_bytes;
             if constexpr (Epi::DIST) { if (p_piece == 0 && epi.route_table() != nullptr) tx += SPMV_ROUTE_WORDS * 4u; }
             mbar_expect_tx(&full[stage], tx);
         }
@@ -334,8 +342,8 @@ inline int pick_lanes(int64_t nnz, int64_t nrows) {
     return L;
 }
 
-inline size_t spmv_smem_bytes(const SpmvPlan& p, int nin, bool route = false) {
-    return (size_t)SPMV_WARPS * p.nst * (spmv_stage_layout(p.cap, p.rw(), nin, route).bytes + 8);
+inline size_t spmv_smem_bytes(const SpmvPlan& p, int nin, bool route = false, int ninb = 0) {
+    return (size_t)SPMV_WARPS * p.nst * (spmv_stage_layout(p.cap, p.rw(), nin, route, ninb).bytes + 8);
 }
 
 // nin_max: the largest operand count among the epilogues that will run with this plan
@@ -374,7 +382,7 @@ template <int L, int RPL, int NSTW, class Epi>
 void launch_spmv_inst(const SpmvPlan& p, int nrows, const int* ptr, const int* idx, const double* val,
                       const double* vec, const Epi& epi, cudaStream_t st) {
     auto kern = spmv_warp_kernel<L, RPL, NSTW, Epi>;
-    const size_t smem = spmv_smem_bytes(p, Epi::NIN, Epi::DIST);
+    const size_t smem = spmv_smem_bytes(p, Epi::NIN, Epi::DIST, Epi::NINB);
     ELP_REQUIRE(smem <= 227 * 1024, "spmv: stage ring of %zu bytes does not fit in shared memory", smem);
     // per device and ring size: raise the dynamic shared-memory limit once and ask how many CTAs really fit
     static size_t cfg_smem[16] = {};
@@ -432,11 +440,17 @@ void launch_spmv(const SpmvPlan& p, int nrows, const int* ptr, const int* idx, c
             return;
         }
     }
-    switch (p.L) {
-        case 1:  launch_spmv_l<1, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
-        case 2:  launch_spmv_l<2, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
-        case 4:  launch_spmv_l<4, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
-        default: launch_spmv_l<8, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
+    if constexpr (Epi::NINB > 0) {   // byte operands: tiles of 16 or 32 rows only
+        ELP_REQUIRE(p.L <= 2, "spmv: an epilogue with byte operands needs a plan of at most two lanes per row (L = %d)", p.L);
+        if (p.L == 1) launch_spmv_l<1, Epi>(p, nrows, ptr, idx, val, vec, epi, st);
+        else launch_spmv_l<2, Epi>(p, nrows, ptr, idx, val, vec, epi, st);
+    } else {
+        switch (p.L) {
+            case 1:  launch_spmv_l<1, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
+            case 2:  launch_spmv_l<2, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
+            case 4:  launch_spmv_l<4, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
+            default: launch_spmv_l<8, Epi>(p, nrows, ptr, idx, val, vec, epi, st); break;
+        }
     }
 }
 
