@@ -40,7 +40,7 @@ class Stats(C.Structure):
                 ("rel_primal_res", C.c_double), ("rel_dual_res", C.c_double), ("rel_gap", C.c_double),
                 ("setup_ms", C.c_double), ("solve_ms", C.c_double), ("total_ms", C.c_double),
                 ("kernel_launches", C.c_int64), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64),
-                ("spmv_ms", C.c_double), ("limit_reached", C.c_int32), ("reserved", C.c_int32)]
+                ("spmv_ms", C.c_double), ("limit_reached", C.c_int32), ("simplex_ctas", C.c_int32)]
 
     def asdict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}

@@ -50,10 +50,10 @@ void pdlp_destroy(Pdlp* p);
 void spmv_host(int m, int n, const int32_t* row_ptr, const int32_t* col_idx, const double* vals, const double* x,
                double* out, const int8_t* sense, const double* rhs, double tol, uint8_t* feasible);
 size_t simplex_smem_bytes(int m, int n);
-void simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
-                          const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
-                          double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model = 0,
-                          int32_t* basis = nullptr);
+int simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
+                         const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
+                         double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model = 0,
+                         int32_t* basis = nullptr);
 void densify_device(int m, int n, const int* ptr, const int* idx, const double* val, double* A, cudaStream_t st);
 void sensitivity(int32_t m, int32_t n, const int32_t* row_ptr, const int32_t* col_idx, const double* vals,
                  const int8_t* sense, const double* rhs, const double* c, int32_t maximize, const double* lb,
@@ -652,8 +652,8 @@ static void solve_small(int32_t m, int32_t n, const int32_t* row_ptr, const int3
     cudaEvent_t e0 = ev.a, e1 = ev.b;
     ELP_CUDA(cudaEventRecord(e0, st));
     densify_device(m, n, ptr.p, idx.p, val.p, A.p, st);
-    simplex_batch_device(1, m, n, A.p, b.p, cd.p, lbd.p, ubd.p, sd.p, maximize, o.max_iter, stat.p, obj.p, xd.p, yd.p,
-                         piv.p, st);
+    const int ctas = simplex_batch_device(1, m, n, A.p, b.p, cd.p, lbd.p, ubd.p, sd.p, maximize, o.max_iter, stat.p, obj.p,
+                                          xd.p, yd.p, piv.p, st);
     ELP_CUDA(cudaEventRecord(e1, st));
     int32_t s = 0, pv = 0;
     stat.download(&s, 1, st); piv.download(&pv, 1, st); obj.download(objval, 1, st); xd.download(x, n, st);
@@ -674,6 +674,7 @@ static void solve_small(int32_t m, int32_t n, const int32_t* row_ptr, const int3
         stats->kernel_launches = g_launches.load() - l0;
         stats->h2d_bytes = nnz * 12 + (int64_t)m * 13 + (int64_t)n * 24;
         stats->d2h_bytes = (int64_t)n * 8 + (int64_t)m * 8 + 16;
+        stats->simplex_ctas = ctas;
     }
 }
 
@@ -928,9 +929,9 @@ int elp_batch_run(elp_batch* hh, const elp_options* opt, elp_stats* stats) {
     EventPair ev;
     cudaEvent_t e0 = ev.a, e1 = ev.b;
     ELP_CUDA(cudaEventRecord(e0, st));
-    simplex_batch_device(h->B, h->m, h->n, h->A.p, h->b.p, h->c.p, h->has_lb ? h->lb.p : nullptr,
-                         h->has_ub ? h->ub.p : nullptr, h->has_sense ? h->sense.p : nullptr, h->maximize, o.max_iter,
-                         h->status.p, h->obj.p, h->x.p, nullptr, h->pivots.p, st);
+    const int ctas = simplex_batch_device(h->B, h->m, h->n, h->A.p, h->b.p, h->c.p, h->has_lb ? h->lb.p : nullptr,
+                                          h->has_ub ? h->ub.p : nullptr, h->has_sense ? h->sense.p : nullptr, h->maximize,
+                                          o.max_iter, h->status.p, h->obj.p, h->x.p, nullptr, h->pivots.p, st);
     ELP_CUDA(cudaEventRecord(e1, st));
     ELP_CUDA(cudaStreamSynchronize(st));
     float ms = 0;
@@ -941,6 +942,7 @@ int elp_batch_run(elp_batch* hh, const elp_options* opt, elp_stats* stats) {
         stats->solve_ms = ms;
         stats->total_ms = wall.ms();
         stats->kernel_launches = g_launches.load() - l0;
+        stats->simplex_ctas = ctas;
     }
     ELP_CATCH
 }
@@ -989,6 +991,7 @@ int elp_solve_batch(int64_t B, int32_t m, int32_t n, const double* A, const doub
     EventPair ev;
     cudaEvent_t e0 = ev.a, e1 = ev.b;
     ELP_CUDA(cudaEventRecord(e0, w.st[0]));
+    int ctas = 0;
     for (int64_t i = 0; i < nchunks; ++i) {
         const int s = (int)(i % BatchStreamWorkspace::NS);
         cudaStream_t st = w.st[s];
@@ -1000,9 +1003,9 @@ int elp_solve_batch(int64_t B, int32_t m, int32_t n, const double* A, const doub
         if (lb) w.lb[s].upload(lb + lo * n, (size_t)cnt * n, st);
         if (ub) w.ub[s].upload(ub + lo * n, (size_t)cnt * n, st);
         if (sense) w.sense[s].upload(sense + lo * m, (size_t)cnt * m, st);
-        simplex_batch_device(cnt, m, n, w.A[s].p, w.b[s].p, w.c[s].p, lb ? w.lb[s].p : nullptr, ub ? w.ub[s].p : nullptr,
-                             sense ? w.sense[s].p : nullptr, maximize, o.max_iter, w.status[s].p, w.obj[s].p, w.x[s].p,
-                             nullptr, w.piv[s].p, st);
+        ctas = simplex_batch_device(cnt, m, n, w.A[s].p, w.b[s].p, w.c[s].p, lb ? w.lb[s].p : nullptr,
+                                    ub ? w.ub[s].p : nullptr, sense ? w.sense[s].p : nullptr, maximize, o.max_iter,
+                                    w.status[s].p, w.obj[s].p, w.x[s].p, nullptr, w.piv[s].p, st);
         w.status[s].download(status + lo, (size_t)cnt, st);
         w.obj[s].download(obj + lo, (size_t)cnt, st);
         w.x[s].download(x + lo * n, (size_t)cnt * n, st);
@@ -1027,6 +1030,7 @@ int elp_solve_batch(int64_t B, int32_t m, int32_t n, const double* A, const doub
         for (int64_t i = 0; i < B; ++i) piv += w.piv_host[i];
         stats->iterations = (int32_t)std::min<int64_t>(piv, 0x7fffffff);
         stats->total_ms = wall.ms();
+        stats->simplex_ctas = ctas;
     }
     ELP_CATCH
 }

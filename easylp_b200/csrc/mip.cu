@@ -7,15 +7,15 @@
 //
 // B200 formulation: the open nodes of the tree are LPs that share A, b, c and the row senses and differ only in the
 // variable bounds, so a whole FRONTIER is one launch of the batched simplex kernel (simplex.cu, shared_model = 1: one
-// LP per warp, the tableau in shared memory; the matrix is read once per node from the L2-resident copy).  The host
+// LP per warp, CTA or cluster, the tableau in shared memory; the matrix is read once per node from the L2-resident copy).  The host
 // keeps the tree: best-bound-first order, up to `wave` nodes per launch, prune by bound against the incumbent,
 // branch on the lowest-indexed fractional integer column (lp_solve's default NODE_FIRSTSELECT) into
 // x_j <= floor(v) and x_j >= ceil(v).  Integrality tolerance 1e-7 (lp_solve's default epsint), pruning gaps 1e-11
 // absolute / 1e-9 relative (lp_solve's default mip_gap).  Status codes are lp_solve's: 0 optimal, 2 unfeasible,
 // 3 unbounded, 1 sub-optimal (a node / time limit stopped the search with an incumbent), 7 timeout (without one).
 //
-// Scope: models whose dense tableau fits one SM's shared memory (the same size rule as the simplex path of
-// elp_solve_lp); larger MILPs are refused with a clear error — the reference's MILPs are tens of variables.
+// Scope: models whose dense tableau fits one SM's shared memory, or beyond that a thread-block cluster of up to 16
+// CTAs (simplex.cu: simplex_ctas decides); larger MILPs are refused with an error naming the shape and the capacity.
 #include "common.cuh"
 #include "../../include/easylp_abi.h"
 #include <algorithm>
@@ -25,11 +25,11 @@
 
 namespace elp {
 
-size_t simplex_smem_bytes(int m, int n);
-void simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
-                          const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
-                          double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model,
-                          int32_t* basis = nullptr);
+int simplex_ctas(int m, int n);
+int simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
+                         const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
+                         double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model,
+                         int32_t* basis = nullptr);
 void densify_device(int m, int n, const int* ptr, const int* idx, const double* val, double* A, cudaStream_t st);
 
 namespace {
@@ -51,9 +51,7 @@ void solve_mip(int32_t m, int32_t n, const int32_t* row_ptr, const int32_t* col_
                const uint8_t* is_int, const elp_options& o, int32_t* status, double* objval, double* x, elp_stats* stats) {
     WallTimer wall;
     const int64_t l0 = g_launches.load();
-    ELP_REQUIRE(simplex_smem_bytes(m, n) <= 200 * 1024,
-                "branch and bound: the dense tableau of a %d x %d model does not fit one SM's shared memory; "
-                "MILPs of this size are outside the GPU path", m, n);
+    const int ctas = simplex_ctas(m, n);       // refuses a tableau larger than the largest cluster before any work
     cudaStream_t st = 0;
     const int64_t nnz = m > 0 ? row_ptr[m] : 0;
     const int WAVE = 4096;
@@ -182,6 +180,7 @@ void solve_mip(int32_t m, int32_t n, const int32_t* row_ptr, const int32_t* col_
         stats->method_used = ELP_METHOD_SIMPLEX;
         stats->iterations = (int32_t)std::min<int64_t>(pivots, 0x7fffffff);
         stats->restarts = (int32_t)std::min<int64_t>(nodes, 0x7fffffff);        // branch-and-bound nodes solved
+        stats->simplex_ctas = ctas;
         stats->primal_obj = *objval;
         stats->dual_obj = *objval;
         stats->solve_ms = dev_ms;

@@ -3,7 +3,8 @@
 // Replaces lpSolveAPI::get.sensitivity.obj / get.sensitivity.rhs behind `$sensitivity_objective` and `$sensitivity_rhs`
 // (/root/reference/R/class.R:613-646: arrays Lower | Current | Upper per variable / per constraint).
 // The LP is solved by the simplex kernel (simplex.cu), which also returns its final basis; the ranging itself is a few
-// dense m x m operations on the host (the models that reach this path fit one SM's shared memory: m is tens of rows):
+// dense operations on the host, O(m^3) for the basis inverse and O(m^2 (m + n)) for the objective ranging (the simplex
+// path takes tableaus up to one thread-block cluster's shared memory, a few hundred rows):
 //   objective ranging  the interval of c_j over which the optimal basis stays optimal (reduced costs keep their sign),
 //   rhs ranging        the interval of b_i over which the optimal basis stays feasible (basic variables keep inside
 //                      their bounds), i.e. over which the dual value of the row is valid.
@@ -18,11 +19,10 @@
 
 namespace elp {
 
-size_t simplex_smem_bytes(int m, int n);
-void simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
-                          const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
-                          double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model,
-                          int32_t* basis);
+int simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
+                         const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
+                         double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model,
+                         int32_t* basis);
 void densify_device(int m, int n, const int* ptr, const int* idx, const double* val, double* A, cudaStream_t st);
 
 // Gauss-Jordan inverse with partial pivoting; returns false when singular
@@ -55,8 +55,6 @@ void sensitivity(int32_t m, int32_t n, const int32_t* row_ptr, const int32_t* co
                  const int8_t* sense, const double* rhs, const double* c, int32_t maximize, const double* lb,
                  const double* ub, const elp_options& o, int32_t* status, double* objval, double* x, double* obj_from,
                  double* obj_till, double* rhs_from, double* rhs_till, double* duals) {
-    ELP_REQUIRE(simplex_smem_bytes(m, n) <= 200 * 1024,
-                "sensitivity: ranging needs the simplex path (a basis); a %d x %d model is solved by PDLP", m, n);
     cudaStream_t st = 0;
     const int64_t nnz = m > 0 ? row_ptr[m] : 0;
     DevBuf<int> ptr((size_t)m + 1), idx(std::max<int64_t>(nnz, 1));

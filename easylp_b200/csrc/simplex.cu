@@ -16,6 +16,7 @@
 #include "common.cuh"
 #include "tma.cuh"
 #include "../../include/easylp_abi.h"
+#include <cooperative_groups.h>
 #include <algorithm>
 #include <cmath>
 
@@ -752,6 +753,373 @@ simplex_warp_kernel(int64_t B, int m, int n, const double* __restrict__ Ag, cons
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Cluster kernel for tableaus beyond one SM: one LP per thread-block cluster of C CTAs (C = 2, 4, 8, 16), the
+// tableau spread over the cluster's distributed shared memory.  Same algorithm, tolerances and pivot limit as
+// simplex_batch_kernel.
+//   column slices   CTA k owns the columns [k w, (k+1) w) of [A | I] for all m rows, and their lo, hi, cost, xn,
+//                   state and pivot-row entries;
+//   replicated rows every CTA keeps beta, basis, cb, colq and the bounds and cost of each row's basic variable;
+//   per pivot       pricing over the own columns + a cluster argmax of (value, index) (exchange 1: each CTA
+//                   stores its candidate into every peer), then the owner of the entering column q stores colq and
+//                   q's scalars into every peer (exchange 2); the ratio test runs redundantly on the replicated rows
+//                   (same result everywhere, no exchange), the pivot row and the rank-1 update are local.
+// Two cluster barriers per pivot, no global memory inside the loop.  Determinism: every column's reduced cost,
+// pivot-row entry and update is the CTA kernel's expression with the same sequential loop over i; the argmax /
+// argmin order (value, then smallest index) is total, so the cluster reduction picks the CTA kernel's q and r.
+// Status, pivots, basis, x and y are therefore the CTA kernel's bytes; the objective's final sum is ordered
+// differently (one partial per CTA).  beta = b - A xN is formed by every CTA from global memory with the CTA
+// kernel's loop over j, so the replicated rows start identical in every CTA.
+// ------------------------------------------------------------------------------------------------
+constexpr int SC_THREADS = 256;
+constexpr int SC_MAX_CTAS = 16;
+constexpr size_t SC_SMEM_MAX = 227 * 1024;
+
+// Per-CTA shared memory of the cluster kernel.  w = ceil((m + n) / C) rounded up to even (16-byte rows for the
+// bulk copies).  Bytes = 8 m w (tableau slice) + 44 w (lo hi cost xn rowr, state) + 52 m (beta blo bhi bcost cb
+// colq, basis; m rounded up to even / to 4) + 368 (reduction scratch, exchange slots, q's scalars, mbarrier).
+struct ClusterSimplexLayout {
+    int m, n, N, C, w;
+    size_t off_T, off_beta, off_blo, off_bhi, off_bcost, off_cb, off_colq, off_lo, off_hi, off_cost, off_xn, off_rowr,
+        off_redv, off_slotv, off_objv, off_q, off_bar, off_basis, off_state, off_redi, off_sloti, off_qstate, total;
+    __host__ __device__ ClusterSimplexLayout(int m_, int n_, int C_) : m(m_), n(n_), N(m_ + n_), C(C_) {
+        w = (((N + C - 1) / C) + 1) & ~1;
+        auto up2 = [](size_t v) { return (v + 1) & ~(size_t)1; };
+        size_t o = 0;
+        off_T = o;     o += (size_t)m * w;
+        off_beta = o;  o += up2(m);
+        off_blo = o;   o += up2(m);
+        off_bhi = o;   o += up2(m);
+        off_bcost = o; o += up2(m);
+        off_cb = o;    o += up2(m);
+        off_colq = o;  o += up2(m);
+        off_lo = o;    o += w;
+        off_hi = o;    o += w;
+        off_cost = o;  o += w;
+        off_xn = o;    o += w;
+        off_rowr = o;  o += w;
+        off_redv = o;  o += 8;
+        off_slotv = o; o += SC_MAX_CTAS;
+        off_objv = o;  o += SC_MAX_CTAS;
+        off_q = o;     o += 4;
+        size_t bytes = o * sizeof(double);
+        off_bar = bytes;    bytes += 16;
+        off_basis = bytes;  bytes += (size_t)((m + 3) & ~3) * sizeof(int);
+        off_state = bytes;  bytes += (size_t)((w + 3) & ~3) * sizeof(int);
+        off_redi = bytes;   bytes += 8 * sizeof(int);
+        off_sloti = bytes;  bytes += SC_MAX_CTAS * sizeof(int);
+        off_qstate = bytes; bytes += 4 * sizeof(int);
+        total = bytes;
+    }
+};
+
+__device__ __forceinline__ double start_value(const double* lb, const double* ub, int j) {   // xn of a column at setup
+    const double l = lb ? lb[j] : 0.0, u = ub ? ub[j] : INFINITY;
+    return isfinite(l) ? l : (isfinite(u) ? u : 0.0);
+}
+
+__global__ void __launch_bounds__(SC_THREADS)
+simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict__ Ag, const double* __restrict__ bg,
+                       const double* __restrict__ cg_, const double* __restrict__ lbg, const double* __restrict__ ubg,
+                       const int8_t* __restrict__ senseg, int maximize, int max_pivots, int shared_model,
+                       int32_t* __restrict__ status_out, double* __restrict__ obj_out, double* __restrict__ x_out,
+                       double* __restrict__ y_out, int32_t* __restrict__ pivots_out, int32_t* __restrict__ basis_out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    namespace cgr = cooperative_groups;
+    cgr::cluster_group cluster = cgr::this_cluster();
+    constexpr int T = SC_THREADS;
+    const ClusterSimplexLayout lay(m, n, C);
+    const int N = lay.N, w = lay.w;
+    double* sd = reinterpret_cast<double*>(smem_raw);
+    double* Tl = sd + lay.off_T;                 // [m][w]: my columns of [A | I]
+    double* beta = sd + lay.off_beta;
+    double* blo = sd + lay.off_blo;              // bounds and cost of row i's basic variable
+    double* bhi = sd + lay.off_bhi;
+    double* bcost = sd + lay.off_bcost;
+    double* cb = sd + lay.off_cb;
+    double* colq = sd + lay.off_colq;
+    double* lo = sd + lay.off_lo;                // [w]: scalars of my columns
+    double* hi = sd + lay.off_hi;
+    double* cost = sd + lay.off_cost;
+    double* xn = sd + lay.off_xn;
+    double* rowr = sd + lay.off_rowr;
+    double* red_v = sd + lay.off_redv;
+    double* slot_v = sd + lay.off_slotv;         // exchange 1: one candidate per CTA
+    double* obj_v = sd + lay.off_objv;           // objective partials (rank 0)
+    double* qv = sd + lay.off_q;                 // exchange 2: lo, hi, xn, cost of the entering column
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + lay.off_bar);
+    int* basis = reinterpret_cast<int*>(smem_raw + lay.off_basis);
+    int* state = reinterpret_cast<int*>(smem_raw + lay.off_state);
+    int* red_i = reinterpret_cast<int*>(smem_raw + lay.off_redi);
+    int* slot_i = reinterpret_cast<int*>(smem_raw + lay.off_sloti);
+    int* qstate = reinterpret_cast<int*>(smem_raw + lay.off_qstate);
+    const int tid = threadIdx.x;
+    const int rank = (int)cluster.block_rank();
+    const int j0 = rank * w;                                   // global id of my first column
+    const int ns = min(max(n - j0, 0), w);                     // structural columns in my slice
+
+    const int64_t lp = (int64_t)blockIdx.x / C;
+    const int64_t mlp = shared_model ? 0 : lp;
+    const double* A = Ag + mlp * (int64_t)m * n;
+    const double* b = bg + mlp * (int64_t)m;
+    const double* c = cg_ + mlp * (int64_t)n;
+    const double* lb = lbg ? lbg + lp * (int64_t)n : nullptr;
+    const double* ub = ubg ? ubg + lp * (int64_t)n : nullptr;
+    const int8_t* sense = senseg ? senseg + mlp * (int64_t)m : nullptr;
+
+    // ---- stage my slice: one bulk copy per row segment where alignment allows, cooperative loads otherwise -----
+    const bool tA = m > 0 && ns > 0 && (ns % 2 == 0) && (n % 2 == 0) && ((((uintptr_t)A) & 15) == 0);
+    if (tid == 0) { mbar_init(bar, 1); mbar_fence_init(); }
+    __syncthreads();
+    if (tA) {
+        if (tid == 0) mbar_expect_tx(bar, (uint32_t)m * (uint32_t)ns * 8u);
+        __syncthreads();
+        for (int i = tid; i < m; i += T) tma_load_1d(Tl + (size_t)i * w, A + (size_t)i * n + j0, (uint32_t)ns * 8u, bar);
+    } else {
+        for (int e = tid; e < m * ns; e += T) { const int i = e / ns, jl = e - i * ns; Tl[i * w + jl] = A[(size_t)i * n + j0 + jl]; }
+    }
+    if (ns < w)      // slack columns (identity) and padding (zero)
+        for (int e = tid; e < m * (w - ns); e += T) {
+            const int i = e / (w - ns), jl = ns + (e - i * (w - ns)), j = j0 + jl;
+            Tl[i * w + jl] = (j < N && j - n == i) ? 1.0 : 0.0;
+        }
+    for (int jl = tid; jl < w; jl += T) {
+        const int j = j0 + jl;
+        if (j < n) {
+            const double l = lb ? lb[j] : 0.0, u = ub ? ub[j] : INFINITY;
+            lo[jl] = l; hi[jl] = u;
+            cost[jl] = maximize ? -c[j] : c[j];
+            if (isfinite(l)) { state[jl] = ST_LOWER; xn[jl] = l; }
+            else if (isfinite(u)) { state[jl] = ST_UPPER; xn[jl] = u; }
+            else { state[jl] = ST_FREE; xn[jl] = 0.0; }
+        } else if (j < N) {
+            const int s = sense ? sense[j - n] : 0;
+            lo[jl] = (s == ELP_GE) ? -INFINITY : 0.0;
+            hi[jl] = (s == ELP_LE) ? INFINITY : 0.0;
+            cost[jl] = 0.0; xn[jl] = 0.0; state[jl] = ST_BASIC;
+        } else {
+            lo[jl] = 0.0; hi[jl] = 0.0; cost[jl] = 0.0; xn[jl] = 0.0; state[jl] = ST_BASIC;
+        }
+        rowr[jl] = 0.0;
+    }
+    int bad = 0;
+    for (int j = tid; j < n; j += T) {
+        const double l = lb ? lb[j] : 0.0, u = ub ? ub[j] : INFINITY;
+        if (l > u) bad = 1;
+    }
+    bad = __syncthreads_or(bad);
+    // replicated rows; beta = b - A xN with the CTA kernel's loop over j, read from global memory
+    for (int i = tid; i < m; i += T) {
+        const int s = sense ? sense[i] : 0;
+        blo[i] = (s == ELP_GE) ? -INFINITY : 0.0;
+        bhi[i] = (s == ELP_LE) ? INFINITY : 0.0;
+        bcost[i] = 0.0;
+        basis[i] = n + i;
+        const double* Ai = A + (size_t)i * n;
+        double r = b[i];
+        for (int j = 0; j < n; ++j) r -= Ai[j] * start_value(lb, ub, j);
+        beta[i] = r;
+    }
+    if (tA) mbar_wait(bar, 0);
+    cluster.sync();       // every CTA of the cluster is running and staged before any peer store
+
+    int status = ELP_STATUS_TIMEOUT, pivots = 0, degenerate_run = 0, bland = 0;
+    int qfinal = -1;
+    if (max_pivots <= 0) max_pivots = 50 * (m + n) + 1000;
+    if (bad) status = ELP_STATUS_INFEASIBLE;
+
+    while (!bad) {
+        // ---- phase detection (replicated rows): phase 1 iff some basic variable is outside its bounds ----------
+        int infeasible = 0;
+        for (int i = tid; i < m; i += T) {
+            const double bi = beta[i], l = blo[i], u = bhi[i];
+            double g = 0.0;
+            if (bi < l - ptol(l)) g = -1.0;
+            else if (bi > u + ptol(u)) g = 1.0;
+            cb[i] = g;
+            infeasible |= (g != 0.0);
+        }
+        const bool phase1 = __syncthreads_or(infeasible);
+        if (!phase1) for (int i = tid; i < m; i += T) cb[i] = bcost[i];
+        __syncthreads();
+        // ---- pricing over my columns, then the cluster argmax (exchange 1) ---------------------------------------
+        ValIdx cand{0.0, -1};
+        for (int jl = tid; jl < w; jl += T) {
+            const int st = state[jl];
+            if (st == ST_BASIC || !(lo[jl] < hi[jl])) continue;
+            double d = phase1 ? 0.0 : cost[jl];
+            for (int i = 0; i < m; ++i) d -= cb[i] * Tl[i * w + jl];
+            int dd = 0;
+            if ((st == ST_LOWER || st == ST_FREE) && d < -TOL_DUAL) dd = 1;
+            else if ((st == ST_UPPER || st == ST_FREE) && d > TOL_DUAL) dd = -1;
+            if (!dd) continue;
+            const int j = j0 + jl;
+            ValIdx me{bland ? -(double)j : fabs(d), 2 * j + (dd < 0 ? 1 : 0)};
+            cand = better(cand, me);
+        }
+        cand = block_argmax<T>(cand, red_v, red_i);
+        if (tid < C) {
+            cluster.map_shared_rank(slot_v, tid)[rank] = cand.v;
+            cluster.map_shared_rank(slot_i, tid)[rank] = cand.i;
+        }
+        cluster.sync();
+        cand = ValIdx{slot_v[0], slot_i[0]};
+        for (int k = 1; k < C; ++k) cand = better(cand, ValIdx{slot_v[k], slot_i[k]});
+        if (cand.i < 0) { status = phase1 ? ELP_STATUS_INFEASIBLE : ELP_STATUS_OPTIMAL; break; }
+        if (pivots >= max_pivots) { status = ELP_STATUS_TIMEOUT; break; }
+        const int q = cand.i >> 1;
+        const double dir = (cand.i & 1) ? -1.0 : 1.0;
+        const int qo = q / w, ql = q - qo * w;
+        // ---- entering column: its owner stores colq and q's scalars into every CTA (exchange 2) ------------------
+        if (rank == qo) {
+            for (int k = 0; k < C; ++k) {
+                double* dst = cluster.map_shared_rank(colq, k);
+                for (int i = tid; i < m; i += T) dst[i] = Tl[i * w + ql];
+            }
+            if (tid < C) {
+                double* dq = cluster.map_shared_rank(qv, tid);
+                dq[0] = lo[ql]; dq[1] = hi[ql]; dq[2] = xn[ql]; dq[3] = cost[ql];
+                cluster.map_shared_rank(qstate, tid)[0] = state[ql];
+            }
+        }
+        cluster.sync();
+        const double q_lo = qv[0], q_hi = qv[1], q_xn = qv[2], q_cost = qv[3];
+        const int q_state = qstate[0];
+        // ---- ratio test, pass 1 (replicated) ----------------------------------------------------------------------
+        double tloc = INFINITY;
+        for (int i = tid; i < m; i += T) {
+            const double a = dir * colq[i];
+            if (fabs(a) <= TOL_PIVOT) continue;
+            const double bi = beta[i], l = blo[i], u = bhi[i];
+            double t = INFINITY;
+            if (a > 0.0) {
+                if (bi > u + ptol(u)) t = (bi - u) / a;
+                else if (bi >= l - ptol(l)) { if (isfinite(l)) t = fmax(bi - l, 0.0) / a; }
+            } else {
+                if (bi < l - ptol(l)) t = (bi - l) / a;
+                else if (bi <= u + ptol(u)) { if (isfinite(u)) t = fmin(bi - u, 0.0) / a; }
+            }
+            tloc = fmin(tloc, t);
+        }
+        ValIdx tm = block_argmax<T>(ValIdx{-tloc, tid}, red_v, red_i);
+        const double tmin = -tm.v;
+        double tflip = (q_state == ST_FREE) ? INFINITY : q_hi - q_lo;
+        if (tflip <= tmin) {
+            if (!isfinite(tflip)) {
+                if (phase1) { status = ELP_STATUS_NUMFAILURE; break; }
+                status = ELP_STATUS_UNBOUNDED;
+                qfinal = q;
+                __syncthreads();
+                if (tid == 0 && rank == qo) xn[ql] = dir > 0 ? INFINITY : -INFINITY;
+                break;
+            }
+            for (int i = tid; i < m; i += T) beta[i] -= dir * tflip * colq[i];
+            __syncthreads();
+            if (tid == 0 && rank == qo) {
+                if (dir > 0) { state[ql] = ST_UPPER; xn[ql] = hi[ql]; }
+                else { state[ql] = ST_LOWER; xn[ql] = lo[ql]; }
+            }
+            ++pivots; degenerate_run = 0; bland = 0;
+            __syncthreads();
+            continue;
+        }
+        // ---- pass 2: among rows within a hair of tmin take the largest pivot (Bland: smallest basic id) ----------
+        const double window = tmin + 1e-12 * fmax(1.0, fabs(tmin));
+        ValIdx rc{0.0, -1};
+        for (int i = tid; i < m; i += T) {
+            const double a = dir * colq[i];
+            if (fabs(a) <= TOL_PIVOT) continue;
+            const int k = basis[i];
+            const double bi = beta[i], l = blo[i], u = bhi[i];
+            double t = INFINITY; int up = 0;
+            if (a > 0.0) {
+                if (bi > u + ptol(u)) { t = (bi - u) / a; up = 1; }
+                else if (bi >= l - ptol(l)) { if (isfinite(l)) { t = fmax(bi - l, 0.0) / a; up = 0; } }
+            } else {
+                if (bi < l - ptol(l)) { t = (bi - l) / a; up = 0; }
+                else if (bi <= u + ptol(u)) { if (isfinite(u)) { t = fmin(bi - u, 0.0) / a; up = 1; } }
+            }
+            if (t > window) continue;
+            ValIdx me{bland ? -(double)k : fabs(a), 2 * i + up};
+            rc = better(rc, me);
+        }
+        rc = block_argmax<T>(rc, red_v, red_i);
+        if (rc.i < 0) { status = ELP_STATUS_NUMFAILURE; break; }
+        const int r = rc.i >> 1;
+        const int to_upper = rc.i & 1;
+        // ---- step + basis change --------------------------------------------------------------------------------
+        const double t = tmin;
+        const double piv = colq[r];
+        for (int i = tid; i < m; i += T) beta[i] -= dir * t * colq[i];
+        for (int jl = tid; jl < w; jl += T) rowr[jl] = Tl[r * w + jl] / piv;
+        __syncthreads();
+        if (tid == 0) {
+            const int kl = basis[r];
+            if (kl / w == rank) {
+                const int l = kl - j0;
+                if (to_upper) { state[l] = ST_UPPER; xn[l] = hi[l]; }
+                else { state[l] = ST_LOWER; xn[l] = lo[l]; }
+            }
+            beta[r] = q_xn + dir * t;
+            basis[r] = q; blo[r] = q_lo; bhi[r] = q_hi; bcost[r] = q_cost;
+            if (rank == qo) { state[ql] = ST_BASIC; rowr[ql] = 1.0; }
+        }
+        __syncthreads();
+        // ---- rank-1 update of my columns:  T -= colq * rowr  (row r := rowr) -------------------------------------
+        for (int i = 0; i < m; ++i) {
+            const double f = colq[i];
+            if (i == r) {
+                for (int jl = tid; jl < w; jl += T) Tl[i * w + jl] = rowr[jl];
+            } else if (f != 0.0) {
+                for (int jl = tid; jl < w; jl += T) {
+                    double* e = &Tl[i * w + jl];
+                    *e = (j0 + jl == q) ? 0.0 : *e - f * rowr[jl];      // the pivot column becomes a unit vector exactly
+                }
+            }
+        }
+        ++pivots;
+        if (t <= 1e-12) { if (++degenerate_run > 30) bland = 1; }
+        else { degenerate_run = 0; bland = 0; }
+        __syncthreads();
+    }
+    __syncthreads();
+
+    // ---- write back: owners write their non-basic columns and slack duals, rank 0 the replicated rows ----------
+    double* xo = x_out + lp * (int64_t)n;
+    for (int jl = tid; jl < ns; jl += T) if (state[jl] != ST_BASIC) xo[j0 + jl] = xn[jl];
+    if (rank == 0) for (int i = tid; i < m; i += T) if (basis[i] < n) xo[basis[i]] = beta[i];
+    double opart = 0.0;
+    for (int jl = tid; jl < ns; jl += T) {
+        if (state[jl] != ST_BASIC) opart += cost[jl] * ((j0 + jl == qfinal) ? 0.0 : xn[jl]);
+    }
+    if (rank == 0) for (int i = tid; i < m; i += T) if (basis[i] < n) opart += bcost[i] * beta[i];
+    const double part = block_sum<T>(opart, red_v);
+    if (tid == 0) cluster.map_shared_rank(obj_v, 0)[rank] = part;
+    cluster.sync();
+    if (rank == 0) {
+        if (tid == 0) {
+            double obj = 0.0;
+            for (int k = 0; k < C; ++k) obj += obj_v[k];
+            if (status == ELP_STATUS_UNBOUNDED) obj = -INFINITY;
+            status_out[lp] = status;
+            obj_out[lp] = maximize ? -obj : obj;
+            if (pivots_out) pivots_out[lp] = pivots;
+        }
+        if (basis_out)
+            for (int i = tid; i < m; i += T) basis_out[lp * (int64_t)m + i] = basis[i];
+    }
+    if (y_out) {     // y_i = sum_k cost[basis[k]] * T[k][n + i], by the owner of slack column n + i
+        double* yo = y_out + lp * (int64_t)m;
+        for (int jl = tid; jl < w; jl += T) {
+            const int j = j0 + jl;
+            if (j < n || j >= N) continue;
+            double s = 0.0;
+            for (int k = 0; k < m; ++k) s += bcost[k] * Tl[k * w + jl];
+            yo[j - n] = maximize ? -s : s;
+        }
+    }
+}
+
 __global__ void k_densify(int m, int n, const int* __restrict__ ptr, const int* __restrict__ idx,
                           const double* __restrict__ val, double* __restrict__ A) {
     const int i = blockIdx.x;
@@ -821,18 +1189,86 @@ static bool simplex_warp_launch(int64_t B, int m, int n, const double* A, const 
     return false;
 }
 
-// all pointers are device pointers
-void simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
-                          const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
-                          double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model,
-                          int32_t* basis) {
-    if (B <= 0) return;
+// Can the device schedule one cluster of C CTAs with this much shared memory each?  C = 16 is a non-portable size.
+static bool cluster_schedulable(int C, size_t smem) {
+    if (smem > SC_SMEM_MAX) return false;
+    ELP_CUDA(cudaFuncSetAttribute(simplex_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (C > 8) ELP_CUDA(cudaFuncSetAttribute(simplex_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)C);
+    cfg.blockDim = dim3(SC_THREADS);
+    cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = (unsigned)C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    int clusters = 0;
+    if (cudaOccupancyMaxActiveClusters(&clusters, simplex_cluster_kernel, &cfg) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    return clusters >= 1;
+}
+
+// The one place that decides how many CTAs hold one LP's tableau: 1 (the warp kernel, else the CTA kernel: one SM)
+// or C (the cluster kernel, the smallest C in {2, 4, 8, 16} that fits and can be scheduled).  ELP_SIMPLEX_CLUSTER=C
+// forces the cluster kernel with C CTAs on any shape it can hold.  Throws when no kernel can take the shape.
+int simplex_ctas(int m, int n) {
+    const char* e = getenv("ELP_SIMPLEX_CLUSTER");
+    const int forced = e ? atoi(e) : 0;
+    if (forced == 2 || forced == 4 || forced == 8 || forced == 16) {
+        if (cluster_schedulable(forced, ClusterSimplexLayout(m, n, forced).total)) return forced;
+    }
+    if (simplex_smem_bytes(m, n) <= SC_SMEM_MAX) return 1;
+    int largest = 0;
+    for (int C = 2; C <= SC_MAX_CTAS; C *= 2) {
+        if (!cluster_schedulable(C, std::min(ClusterSimplexLayout(m, n, C).total, SC_SMEM_MAX))) continue;
+        largest = C;
+        if (ClusterSimplexLayout(m, n, C).total <= SC_SMEM_MAX) return C;
+    }
+    int ncap = 0;          // structural columns the largest schedulable cluster holds at this row count
+    if (largest) {
+        int lo = 0, hi = 1 << 24;
+        while (lo < hi) {
+            const int mid = lo + (hi - lo + 1) / 2;
+            if (ClusterSimplexLayout(m, mid, largest).total <= SC_SMEM_MAX) lo = mid;
+            else hi = mid - 1;
+        }
+        ncap = lo;
+    }
+    throw Error(format("simplex: the dense tableau [A | I] of a %d x %d model (%lld doubles) exceeds the largest "
+                       "thread-block cluster this device schedules (%d CTAs x 227 KB of shared memory: at %d rows it "
+                       "holds at most %d columns)", m, n, (long long)m * (m + n), largest, m, ncap));
+}
+
+// all pointers are device pointers; returns the CTAs that held each tableau (simplex_ctas)
+int simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
+                         const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
+                         double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model,
+                         int32_t* basis) {
     ELP_REQUIRE(n > 0 && m >= 0, "simplex: bad shape %d x %d", m, n);
-    ELP_REQUIRE(B < 0x7fffffffll, "simplex: batch too large");
-    if (simplex_warp_launch(B, m, n, A, b, c, lb, ub, sense, maximize, max_pivots, status, obj, x, y, pivots, st, shared_model, basis)) return;
+    const int ctas = simplex_ctas(m, n);
+    if (B <= 0) return ctas;
+    ELP_REQUIRE(B * ctas < 0x7fffffffll, "simplex: batch too large");
+    if (ctas > 1) {
+        const size_t smem = ClusterSimplexLayout(m, n, ctas).total;
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)(B * ctas));
+        cfg.blockDim = dim3(SC_THREADS);
+        cfg.dynamicSmemBytes = smem;
+        cfg.stream = st;
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = (unsigned)ctas; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+        cfg.attrs = at; cfg.numAttrs = 1;
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        ELP_CUDA(cudaLaunchKernelEx(&cfg, simplex_cluster_kernel, B, m, n, ctas, A, b, c, lb, ub, sense, maximize,
+                                    max_pivots, shared_model, status, obj, x, y, pivots, basis));
+        ELP_CUDA(cudaGetLastError());
+        return ctas;
+    }
+    if (simplex_warp_launch(B, m, n, A, b, c, lb, ub, sense, maximize, max_pivots, status, obj, x, y, pivots, st, shared_model, basis)) return 1;
     const size_t smem = simplex_smem_bytes(m, n);
-    ELP_REQUIRE(smem <= 227 * 1024, "simplex: tableau of %d x %d needs %zu bytes of shared memory (max 227 KB)", m, n,
-                smem);
     const int threads = simplex_pick_threads(m, n);
 #define ELP_SIMPLEX_LAUNCH(T)                                                                                     \
     do {                                                                                                          \
@@ -845,6 +1281,7 @@ void simplex_batch_device(int64_t B, int m, int n, const double* A, const double
     else if (threads == 64) ELP_SIMPLEX_LAUNCH(64);
     else ELP_SIMPLEX_LAUNCH(128);
 #undef ELP_SIMPLEX_LAUNCH
+    return 1;
 }
 
 void densify_device(int m, int n, const int* ptr, const int* idx, const double* val, double* A, cudaStream_t st) {

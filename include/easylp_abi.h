@@ -39,8 +39,10 @@ extern "C" {
 #define ELP_STATUS_NUMFAILURE 5
 #define ELP_STATUS_TIMEOUT 7
 
-#define ELP_METHOD_AUTO 0    /* size rule: dense tableau fits in shared memory -> simplex, else PDLP */
-#define ELP_METHOD_SIMPLEX 1
+#define ELP_METHOD_AUTO 0    /* size rule: dense tableau fits 200 KB of one SM's shared memory -> simplex, else PDLP */
+#define ELP_METHOD_SIMPLEX 1  /* dense tableau in one SM's shared memory, or beyond that spread over a thread-block
+                                 cluster of 2-16 CTAs (about 420 k tableau entries m (m + n) at 16 CTAs, a few hundred
+                                 rows); larger models are refused with an error naming the shape and the capacity */
 #define ELP_METHOD_PDLP 2
 
 /* How the plain PDHG iterations obtain g = A'y (pdlp.cu).
@@ -92,7 +94,8 @@ typedef struct elp_stats {
     double spmv_ms;            /* device time of the timed A.x / A'.y probe (elp_pdlp_probe_spmv) */
     int32_t limit_reached;     /* with status 7: 0 = only this call's max_new_iters ran out (call again), 1 = the iteration
                                   limit of the solve, 2 = its time limit (lp.control(timeout=)) — do not call again */
-    int32_t reserved;
+    int32_t simplex_ctas;      /* CTAs that held each simplex tableau: 0 PDLP ran, 1 one SM (warp or CTA kernel), C a
+                                  thread-block cluster of C CTAs (tableaus beyond one SM's shared memory) */
 } elp_stats;
 
 /* ---- housekeeping -------------------------------------------------------------------------- */
@@ -208,7 +211,8 @@ int elp_solve_lp(int32_t m, int32_t n,
  *      differ in their bounds: every frontier is ONE launch of the batched simplex kernel (csrc/mip.cu).  Status codes as
  *      lp_solve: 0 optimal, 2 unfeasible, 3 unbounded, 1 sub-optimal / 7 timeout when opt->max_iter (a NODE limit here) or
  *      opt->time_limit_s stops the search with / without an incumbent.  stats->restarts = nodes solved,
- *      stats->iterations = simplex pivots.  Models whose dense tableau does not fit one SM are refused. */
+ *      stats->iterations = simplex pivots.  Models whose dense tableau does not fit one SM run on the cluster kernel
+ *      (ELP_METHOD_SIMPLEX); beyond the largest cluster they are refused. */
 int elp_solve_mip(int32_t m, int32_t n,
                   const int32_t* row_ptr, const int32_t* col_idx, const double* vals,
                   const int8_t* sense, const double* rhs,
@@ -218,8 +222,8 @@ int elp_solve_mip(int32_t m, int32_t n,
                   int32_t* status, double* objval, double* x /* n */, elp_stats* stats /* may be NULL */);
 
 /* ---- (2c) sensitivity ranging: replaces lpSolveAPI::get.sensitivity.obj / get.sensitivity.rhs behind
- *      `$sensitivity_objective` and `$sensitivity_rhs` (R/class.R:613-646).  Solves the LP on the simplex path (the model
- *      must fit it: ranging needs a basis) and returns, per variable, the interval [obj_from, obj_till] of its cost over
+ *      `$sensitivity_objective` and `$sensitivity_rhs` (R/class.R:613-646).  Solves the LP on the simplex path (ranging
+ *      needs a basis; one SM, or a thread-block cluster for larger tableaus, as ELP_METHOD_SIMPLEX) and returns, per variable, the interval [obj_from, obj_till] of its cost over
  *      which the optimal basis stays optimal and, per constraint, the interval [rhs_from, rhs_till] of its right-hand
  *      side over which the basis stays feasible (the dual value `duals[i]` is valid there).  Infinite ends are IEEE
  *      infinities.  Textbook basis-invariance ranges; lp_solve's conventions at degenerate vertices are not pinned
@@ -237,7 +241,7 @@ int elp_sensitivity(int32_t m, int32_t n,
 /* ---- (3) a batch of small dense LPs (BASELINE config 3; additive entry point, SURVEY §0.5) ---
  * A is [B][m][n] row-major, b [B][m], c [B][n], lb/ub [B][n] (NULL => 0 / +Inf), sense [B][m]
  * (NULL => all "<=").  One LP per WARP with the tableau in shared memory (shapes with m > 32 or m + n > 96: one LP
- * per CTA); outputs status[B], obj[B], x[B][n]. */
+ * per CTA; tableaus beyond one SM: one LP per thread-block cluster); outputs status[B], obj[B], x[B][n]. */
 int elp_solve_batch(int64_t B, int32_t m, int32_t n,
                     const double* A, const double* b, const double* c,
                     const double* lb, const double* ub, const int8_t* sense, int32_t maximize,

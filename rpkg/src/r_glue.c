@@ -94,8 +94,8 @@ SEXP easylp_assemble_csr(SEXP term_row, SEXP term_col, SEXP term_val, SEXP m_, S
 /* list(status, objval, x, y, stats) of a solve; x and y are PROTECTed by the caller */
 static SEXP solve_result(int32_t status, double objval, SEXP x, SEXP y, const elp_stats* st) {
     const char* snames[] = {"method", "iterations", "restarts", "rel_primal_res", "rel_dual_res", "rel_gap",
-                            "setup_ms", "solve_ms", "kernel_launches", "h2d_bytes", "d2h_bytes"};
-    SEXP stats = PROTECT(named_list(11, snames));
+                            "setup_ms", "solve_ms", "kernel_launches", "h2d_bytes", "d2h_bytes", "simplex_ctas"};
+    SEXP stats = PROTECT(named_list(12, snames));
     SET_VECTOR_ELT(stats, 0, Rf_ScalarInteger(st->method_used));
     SET_VECTOR_ELT(stats, 1, Rf_ScalarInteger(st->iterations));
     SET_VECTOR_ELT(stats, 2, Rf_ScalarInteger(st->restarts));
@@ -107,6 +107,7 @@ static SEXP solve_result(int32_t status, double objval, SEXP x, SEXP y, const el
     SET_VECTOR_ELT(stats, 8, Rf_ScalarReal((double)st->kernel_launches));
     SET_VECTOR_ELT(stats, 9, Rf_ScalarReal((double)st->h2d_bytes));
     SET_VECTOR_ELT(stats, 10, Rf_ScalarReal((double)st->d2h_bytes));
+    SET_VECTOR_ELT(stats, 11, Rf_ScalarInteger(st->simplex_ctas));
     const char* names[] = {"status", "objval", "x", "y", "stats"};
     SEXP out = PROTECT(named_list(5, names));
     SET_VECTOR_ELT(out, 0, Rf_ScalarInteger(status));
