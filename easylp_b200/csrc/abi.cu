@@ -49,7 +49,7 @@ int pdlp_transpose(Pdlp* p);
 void pdlp_destroy(Pdlp* p);
 void spmv_host(int m, int n, const int32_t* row_ptr, const int32_t* col_idx, const double* vals, const double* x,
                double* out, const int8_t* sense, const double* rhs, double tol, uint8_t* feasible);
-size_t simplex_smem_bytes(int m, int n);
+bool simplex_auto_prefers(int m, int n);
 int simplex_batch_device(int64_t B, int m, int n, const double* A, const double* b, const double* c, const double* lb,
                          const double* ub, const int8_t* sense, int maximize, int max_pivots, int32_t* status,
                          double* obj, double* x, double* y, int32_t* pivots, cudaStream_t st, int shared_model = 0,
@@ -720,7 +720,7 @@ int elp_solve_lp(int32_t m, int32_t n, const int32_t* row_ptr, const int32_t* co
     const elp_options o = effective_options(opt);
     int method = o.method;
     if (method == ELP_METHOD_AUTO)   // size rule, not a backend switch: does the dense tableau fit in one SM?
-        method = (simplex_smem_bytes(m, n) <= 200 * 1024) ? ELP_METHOD_SIMPLEX : ELP_METHOD_PDLP;
+        method = simplex_auto_prefers(m, n) ? ELP_METHOD_SIMPLEX : ELP_METHOD_PDLP;
     // any block with lower > upper forces "unfeasible" (R/class.R:297-298); both solvers also detect it
     if (method == ELP_METHOD_SIMPLEX)
         solve_small(m, n, row_ptr, col_idx, vals, sense, rhs, c, maximize, lb, ub, o, status, objval, x, y, stats);
@@ -867,7 +867,7 @@ int elp_model_solve(const elp_model* hh, const int8_t* sense, const double* rhs,
     const elp_options o = effective_options(opt);
     int method = o.method;
     if (method == ELP_METHOD_AUTO)
-        method = (simplex_smem_bytes(h->m, h->n) <= 200 * 1024) ? ELP_METHOD_SIMPLEX : ELP_METHOD_PDLP;
+        method = simplex_auto_prefers(h->m, h->n) ? ELP_METHOD_SIMPLEX : ELP_METHOD_PDLP;
     if (method == ELP_METHOD_SIMPLEX) {          // a tableau that fits one SM: the few KB of CSR go through the host path
         std::vector<int32_t> rp((size_t)h->m + 1), ci((size_t)std::max<int64_t>(h->nnz, 1));
         std::vector<double> v((size_t)std::max<int64_t>(h->nnz, 1));

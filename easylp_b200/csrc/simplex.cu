@@ -1,13 +1,14 @@
-// simplex.cu — batched dense simplex: one LP per warp (one per CTA for the larger shapes), tableau resident in shared memory.
+// simplex.cu — batched dense simplex: one LP per warp for small shapes, else one LP per CTA or per thread-block cluster;
+// tableau resident in shared memory.
 //
 // Replaces `status <- solve(prob)` (/root/reference/R/class.R:276) for LPs whose dense tableau fits in
-// one SM's shared memory, and is the engine of the additive batch entry point (BASELINE config 3:
+// the shared memory of one SM or of a cluster, and is the engine of the additive batch entry point (BASELINE config 3:
 // 200k LPs of 20x30).  Method: bounded-variable primal simplex on  A x + s = b  with a composite
 // phase 1 (minimise the sum of infeasibilities), Dantzig pricing, a two-pass ratio test and Bland's
 // rule after a run of degenerate pivots.  The CPU restatement is oracle/simplex_ref.c.
 //
-// Data movement: each LP's A (m*n doubles), b, c, lb, ub are read ONCE from HBM with 1-D TMA bulk
-// copies (cp.async.bulk -> mbarrier complete_tx) straight into their shared-memory homes; results
+// Data movement: each LP's A (m*n doubles) is read ONCE from HBM with 1-D TMA bulk copies, one per row
+// (cp.async.bulk -> mbarrier complete_tx), straight into its shared-memory home, b, c, lb, ub by plain loads; results
 // (status, objective, x) are written once.  Everything in between — pricing argmax, ratio-test
 // argmin (warp shuffles), the rank-1 pivot update — runs out of shared memory in fp64.
 // Algorithmic HBM bytes per LP: 8 (m n + m + 3 n) + m   in,   8 (n + 1) + 4   out.
@@ -77,301 +78,6 @@ __device__ __forceinline__ double block_sum(double x, double* red_v) {
     for (int w = 0; w < THREADS / 32; ++w) r += red_v[w];
     return r;
 }
-template <int THREADS>
-__device__ __forceinline__ void block_sync() {
-    if (THREADS == 32) __syncwarp();
-    else __syncthreads();
-}
-
-struct SimplexSmemLayout {
-    int m, n, N;
-    size_t off_TA, off_TS, off_beta, off_lo, off_hi, off_cost, off_xn, off_cb, off_colq, off_rowr, off_redv;
-    size_t off_basis, off_state, off_redi, off_bar, total;
-    __host__ __device__ SimplexSmemLayout(int m_, int n_) : m(m_), n(n_), N(m_ + n_) {
-        auto up2 = [](size_t v) { return (v + 1) & ~(size_t)1; };   // keep every double array 16B aligned
-        size_t o = 0;
-        off_TA = o;   o += up2((size_t)m * n);
-        off_TS = o;   o += up2((size_t)m * m);
-        off_beta = o; o += up2(m);
-        off_lo = o;   o += up2(N);
-        off_hi = o;   o += up2(N);
-        off_cost = o; o += up2(N);
-        off_xn = o;   o += up2(N);
-        off_cb = o;   o += up2(m);
-        off_colq = o; o += up2(m);
-        off_rowr = o; o += up2(N);
-        off_redv = o; o += 8;
-        size_t bytes = o * sizeof(double);
-        off_bar = bytes;   bytes += 16;
-        off_basis = bytes; bytes += (size_t)((m + 3) & ~3) * sizeof(int);
-        off_state = bytes; bytes += (size_t)((N + 3) & ~3) * sizeof(int);
-        off_redi = bytes;  bytes += 8 * sizeof(int);
-        total = bytes;
-    }
-};
-
-template <int THREADS>
-__global__ void __launch_bounds__(THREADS)
-simplex_batch_kernel(int64_t B, int m, int n, const double* __restrict__ Ag, const double* __restrict__ bg,
-                     const double* __restrict__ cg, const double* __restrict__ lbg, const double* __restrict__ ubg,
-                     const int8_t* __restrict__ senseg, int maximize, int max_pivots, int shared_model,
-                     int32_t* __restrict__ status_out,
-                     double* __restrict__ obj_out, double* __restrict__ x_out, double* __restrict__ y_out,
-                     int32_t* __restrict__ pivots_out, int32_t* __restrict__ basis_out) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const SimplexSmemLayout lay(m, n);
-    const int N = lay.N;
-    double* sd = reinterpret_cast<double*>(smem_raw);
-    double* TA = sd + lay.off_TA;
-    double* TS = sd + lay.off_TS;
-    double* beta = sd + lay.off_beta;
-    double* lo = sd + lay.off_lo;
-    double* hi = sd + lay.off_hi;
-    double* cost = sd + lay.off_cost;
-    double* xn = sd + lay.off_xn;
-    double* cb = sd + lay.off_cb;
-    double* colq = sd + lay.off_colq;
-    double* rowr = sd + lay.off_rowr;
-    double* red_v = sd + lay.off_redv;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + lay.off_bar);
-    int* basis = reinterpret_cast<int*>(smem_raw + lay.off_basis);
-    int* state = reinterpret_cast<int*>(smem_raw + lay.off_state);
-    int* red_i = reinterpret_cast<int*>(smem_raw + lay.off_redi);
-    const int tid = threadIdx.x;
-
-    const int64_t lp = blockIdx.x;
-    if (lp >= B) return;
-    const int64_t mlp = shared_model ? 0 : lp;      // branch and bound: every node shares A, b, c, sense; bounds differ
-    const double* A = Ag + mlp * (int64_t)m * n;
-    const double* b = bg + mlp * (int64_t)m;
-    const double* c = cg + mlp * (int64_t)n;
-    const double* lb = lbg ? lbg + lp * (int64_t)n : nullptr;
-    const double* ub = ubg ? ubg + lp * (int64_t)n : nullptr;
-    const int8_t* sense = senseg ? senseg + mlp * (int64_t)m : nullptr;
-
-    // ---- stage the LP: TMA bulk copies where alignment allows, cooperative loads otherwise ----------
-    const size_t bytesA = (size_t)m * n * 8, bytesb = (size_t)m * 8, bytesn = (size_t)n * 8;
-    const bool tA = tma_ok(A, bytesA), tb = tma_ok(b, bytesb), tc = tma_ok(c, bytesn);
-    const bool tl = lb && tma_ok(lb, bytesn), tu = ub && tma_ok(ub, bytesn);
-    if (tid == 0) { mbar_init(bar, 1); mbar_fence_init(); }
-    block_sync<THREADS>();
-    if (tid == 0) {
-        const uint32_t tx = (uint32_t)((tA ? bytesA : 0) + (tb ? bytesb : 0) + (tc ? bytesn : 0) + (tl ? bytesn : 0) +
-                                       (tu ? bytesn : 0));
-        mbar_expect_tx(bar, tx);
-        if (tA) tma_load_1d(TA, A, (uint32_t)bytesA, bar);
-        if (tb) tma_load_1d(beta, b, (uint32_t)bytesb, bar);
-        if (tc) tma_load_1d(cost, c, (uint32_t)bytesn, bar);
-        if (tl) tma_load_1d(lo, lb, (uint32_t)bytesn, bar);
-        if (tu) tma_load_1d(hi, ub, (uint32_t)bytesn, bar);
-    }
-    // meanwhile: everything that does not depend on the copies
-    for (int e = tid; e < m * m; e += THREADS) TS[e] = (e / m == e % m) ? 1.0 : 0.0;
-    if (!tA) for (int e = tid; e < m * n; e += THREADS) TA[e] = A[e];
-    if (!tb) for (int i = tid; i < m; i += THREADS) beta[i] = b[i];
-    if (!tc) for (int j = tid; j < n; j += THREADS) cost[j] = c[j];
-    if (!tl) for (int j = tid; j < n; j += THREADS) lo[j] = lb ? lb[j] : 0.0;
-    if (!tu) for (int j = tid; j < n; j += THREADS) hi[j] = ub ? ub[j] : INFINITY;
-    for (int i = tid; i < m; i += THREADS) {
-        const int s = sense ? sense[i] : 0;
-        lo[n + i] = (s == ELP_GE) ? -INFINITY : 0.0;
-        hi[n + i] = (s == ELP_LE) ? INFINITY : 0.0;
-        cost[n + i] = 0.0;
-        xn[n + i] = 0.0;
-        state[n + i] = ST_BASIC;
-        basis[i] = n + i;
-    }
-    mbar_wait(bar, 0);
-    block_sync<THREADS>();
-
-    int bad = 0;
-    for (int j = tid; j < n; j += THREADS) {
-        if (maximize) cost[j] = -cost[j];
-        const double l = lo[j], u = hi[j];
-        if (l > u) bad = 1;
-        if (isfinite(l)) { state[j] = ST_LOWER; xn[j] = l; }
-        else if (isfinite(u)) { state[j] = ST_UPPER; xn[j] = u; }
-        else { state[j] = ST_FREE; xn[j] = 0.0; }
-    }
-    bad = __syncthreads_or(bad);
-    // beta = b - A xN
-    for (int i = tid; i < m; i += THREADS) {
-        double r = beta[i];
-        for (int j = 0; j < n; ++j) r -= TA[i * n + j] * xn[j];
-        beta[i] = r;
-    }
-    block_sync<THREADS>();
-
-    int status = ELP_STATUS_TIMEOUT, pivots = 0, degenerate_run = 0, bland = 0;
-    int qfinal = -1;
-    if (max_pivots <= 0) max_pivots = 50 * (m + n) + 1000;
-    if (bad) status = ELP_STATUS_INFEASIBLE;
-
-    while (!bad) {
-        // ---- phase detection ------------------------------------------------------------------
-        double wpart = 0.0;
-        for (int i = tid; i < m; i += THREADS) {
-            const int k = basis[i];
-            const double bi = beta[i];
-            double g = 0.0;
-            if (bi < lo[k] - ptol(lo[k])) { g = -1.0; wpart += lo[k] - bi; }
-            else if (bi > hi[k] + ptol(hi[k])) { g = 1.0; wpart += bi - hi[k]; }
-            cb[i] = g;
-        }
-        const double w = block_sum<THREADS>(wpart, red_v);
-        const bool phase1 = w > 0.0;
-        if (!phase1) for (int i = tid; i < m; i += THREADS) cb[i] = cost[basis[i]];
-        block_sync<THREADS>();
-        // ---- pricing: d_j = cost_j - cb' T[:,j]; Dantzig (largest |d_j|) or Bland (smallest j) ----
-        ValIdx cand{0.0, -1};
-        for (int j = tid; j < N; j += THREADS) {
-            const int st = state[j];
-            if (st == ST_BASIC || !(lo[j] < hi[j])) continue;
-            double d = phase1 ? 0.0 : cost[j];
-            if (j < n) { for (int i = 0; i < m; ++i) d -= cb[i] * TA[i * n + j]; }
-            else { const int jj = j - n; for (int i = 0; i < m; ++i) d -= cb[i] * TS[i * m + jj]; }
-            int dd = 0;
-            if ((st == ST_LOWER || st == ST_FREE) && d < -TOL_DUAL) dd = 1;
-            else if ((st == ST_UPPER || st == ST_FREE) && d > TOL_DUAL) dd = -1;
-            if (!dd) continue;
-            // encode the direction in the index: idx = 2*j + (dd<0)
-            ValIdx me{bland ? -(double)j : fabs(d), 2 * j + (dd < 0 ? 1 : 0)};
-            cand = better(cand, me);
-        }
-        cand = block_argmax<THREADS>(cand, red_v, red_i);
-        if (cand.i < 0) { status = phase1 ? ELP_STATUS_INFEASIBLE : ELP_STATUS_OPTIMAL; break; }
-        if (pivots >= max_pivots) { status = ELP_STATUS_TIMEOUT; break; }
-        const int q = cand.i >> 1;
-        const double dir = (cand.i & 1) ? -1.0 : 1.0;
-        // ---- entering column ------------------------------------------------------------------
-        for (int i = tid; i < m; i += THREADS) colq[i] = (q < n) ? TA[i * n + q] : TS[i * m + (q - n)];
-        block_sync<THREADS>();
-        // ---- ratio test, pass 1: the minimum step (warp-shuffle argmin) ----------------------------
-        double tloc = INFINITY;
-        for (int i = tid; i < m; i += THREADS) {
-            const double a = dir * colq[i];
-            if (fabs(a) <= TOL_PIVOT) continue;
-            const int k = basis[i];
-            const double bi = beta[i], l = lo[k], u = hi[k];
-            double t = INFINITY;
-            if (a > 0.0) {
-                if (bi > u + ptol(u)) t = (bi - u) / a;
-                else if (bi >= l - ptol(l)) { if (isfinite(l)) t = fmax(bi - l, 0.0) / a; }
-            } else {
-                if (bi < l - ptol(l)) t = (bi - l) / a;
-                else if (bi <= u + ptol(u)) { if (isfinite(u)) t = fmin(bi - u, 0.0) / a; }
-            }
-            tloc = fmin(tloc, t);
-        }
-        ValIdx tm = block_argmax<THREADS>(ValIdx{-tloc, tid}, red_v, red_i);
-        const double tmin = -tm.v;
-        double tflip = (state[q] == ST_FREE) ? INFINITY : hi[q] - lo[q];
-        if (tflip <= tmin) {
-            if (!isfinite(tflip)) {
-                if (phase1) { status = ELP_STATUS_NUMFAILURE; break; }
-                status = ELP_STATUS_UNBOUNDED;
-                qfinal = q;
-                block_sync<THREADS>();
-                if (tid == 0) xn[q] = dir > 0 ? INFINITY : -INFINITY;
-                break;
-            }
-            for (int i = tid; i < m; i += THREADS) beta[i] -= dir * tflip * colq[i];
-            block_sync<THREADS>();
-            if (tid == 0) {
-                if (dir > 0) { state[q] = ST_UPPER; xn[q] = hi[q]; }
-                else { state[q] = ST_LOWER; xn[q] = lo[q]; }
-            }
-            ++pivots; degenerate_run = 0; bland = 0;
-            block_sync<THREADS>();
-            continue;
-        }
-        // ---- pass 2: among rows within a hair of tmin take the largest pivot (Bland: smallest basic id) ----
-        const double window = tmin + 1e-12 * fmax(1.0, fabs(tmin));
-        ValIdx rc{0.0, -1};
-        for (int i = tid; i < m; i += THREADS) {
-            const double a = dir * colq[i];
-            if (fabs(a) <= TOL_PIVOT) continue;
-            const int k = basis[i];
-            const double bi = beta[i], l = lo[k], u = hi[k];
-            double t = INFINITY; int up = 0;
-            if (a > 0.0) {
-                if (bi > u + ptol(u)) { t = (bi - u) / a; up = 1; }
-                else if (bi >= l - ptol(l)) { if (isfinite(l)) { t = fmax(bi - l, 0.0) / a; up = 0; } }
-            } else {
-                if (bi < l - ptol(l)) { t = (bi - l) / a; up = 0; }
-                else if (bi <= u + ptol(u)) { if (isfinite(u)) { t = fmin(bi - u, 0.0) / a; up = 1; } }
-            }
-            if (t > window) continue;
-            ValIdx me{bland ? -(double)k : fabs(a), 2 * i + up};
-            rc = better(rc, me);
-        }
-        rc = block_argmax<THREADS>(rc, red_v, red_i);
-        if (rc.i < 0) { status = ELP_STATUS_NUMFAILURE; break; }
-        const int r = rc.i >> 1;
-        const int to_upper = rc.i & 1;
-        // ---- step + basis change --------------------------------------------------------------
-        const double t = tmin;
-        const double piv = colq[r];
-        for (int i = tid; i < m; i += THREADS) beta[i] -= dir * t * colq[i];
-        for (int j = tid; j < N; j += THREADS) rowr[j] = ((j < n) ? TA[r * n + j] : TS[r * m + (j - n)]) / piv;
-        block_sync<THREADS>();
-        if (tid == 0) {
-            const int kl = basis[r];
-            if (to_upper) { state[kl] = ST_UPPER; xn[kl] = hi[kl]; }
-            else { state[kl] = ST_LOWER; xn[kl] = lo[kl]; }
-            beta[r] = xn[q] + dir * t;
-            basis[r] = q;
-            state[q] = ST_BASIC;
-            rowr[q] = 1.0;
-        }
-        block_sync<THREADS>();
-        // ---- rank-1 update of the tableau:  T -= colq * rowr  (row r := rowr) ----------------------
-        for (int i = 0; i < m; ++i) {
-            const double f = colq[i];
-            if (i == r) {
-                for (int j = tid; j < N; j += THREADS) { if (j < n) TA[i * n + j] = rowr[j]; else TS[i * m + (j - n)] = rowr[j]; }
-            } else if (f != 0.0) {
-                for (int j = tid; j < N; j += THREADS) {
-                    double* e = (j < n) ? &TA[i * n + j] : &TS[i * m + (j - n)];
-                    *e = (j == q) ? 0.0 : *e - f * rowr[j];      // the pivot column becomes a unit vector exactly
-                }
-            }
-        }
-        ++pivots;
-        if (t <= 1e-12) { if (++degenerate_run > 30) bland = 1; }
-        else { degenerate_run = 0; bland = 0; }
-        block_sync<THREADS>();
-    }
-    block_sync<THREADS>();
-
-    // ---- write back ---------------------------------------------------------------------------
-    double* xo = x_out + lp * (int64_t)n;
-    for (int j = tid; j < n; j += THREADS) if (state[j] != ST_BASIC) xo[j] = xn[j];
-    for (int i = tid; i < m; i += THREADS) if (basis[i] < n) xo[basis[i]] = beta[i];
-    double opart = 0.0;
-    for (int j = tid; j < n; j += THREADS) {
-        if (state[j] != ST_BASIC) opart += cost[j] * ((j == qfinal) ? 0.0 : xn[j]);
-    }
-    for (int i = tid; i < m; i += THREADS) if (basis[i] < n) opart += cost[basis[i]] * beta[i];
-    double obj = block_sum<THREADS>(opart, red_v);
-    if (status == ELP_STATUS_UNBOUNDED) obj = -INFINITY;
-    if (tid == 0) {
-        status_out[lp] = status;
-        obj_out[lp] = maximize ? -obj : obj;
-        if (pivots_out) pivots_out[lp] = pivots;
-    }
-    if (basis_out)      // final basis, one column id per row (structural j < n, slack of row i = n + i): sensitivity ranging
-        for (int i = tid; i < m; i += THREADS) basis_out[lp * (int64_t)m + i] = basis[i];
-    if (y_out) {
-        double* yo = y_out + lp * (int64_t)m;
-        for (int i = tid; i < m; i += THREADS) {
-            double s = 0.0;
-            for (int k = 0; k < m; ++k) s += cost[basis[k]] * TS[k * m + i];
-            yo[i] = maximize ? -s : s;
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------------------------
 // Warp-per-LP kernel for small LPs (m <= 32, m + n <= 96) — the batched path of BASELINE config 3.
 // One WARP solves one LP; a CTA is four independent warps.  The tableau T[MR][NS] (NS = 32*CPL + 2 doubles
@@ -387,7 +93,7 @@ simplex_batch_kernel(int64_t B, int m, int n, const double* __restrict__ Ag, con
 //   update      T[i][j] -= colq[i] * rr[j]: MR fused multiply-adds per column straight on shared memory;
 //               the dynamic pivot row is a plain address here (registers could not be indexed by it)
 // There is no block-wide barrier, no address arithmetic in the loops and ~60 registers per thread, so many
-// LPs are resident per SM.  Arithmetic order per entry equals simplex_batch_kernel / oracle/simplex_ref.c.
+// LPs are resident per SM.  Arithmetic order per entry equals simplex_kernel / oracle/simplex_ref.c.
 // ------------------------------------------------------------------------------------------------
 constexpr int SW_WARPS = 4;
 
@@ -407,7 +113,7 @@ struct WVI {
     int i;
 };
 // Warp argmax of (v, i) with v >= 0 (or i < 0 = no candidate): larger v wins, ties go to the smaller i — the
-// "better" of simplex_batch_kernel.  Non-negative doubles order like their bit patterns, so the maximum is two
+// "better" above.  Non-negative doubles order like their bit patterns, so the maximum is two
 // 32-bit hardware reductions (REDUX) on the high and low words and the tie-break a third on the index.
 __device__ __forceinline__ WVI warp_best_nonneg(WVI x) {
     const unsigned long long bits = x.i < 0 ? 0ull : (unsigned long long)__double_as_longlong(x.v + 0.0);
@@ -754,35 +460,36 @@ simplex_warp_kernel(int64_t B, int m, int n, const double* __restrict__ Ag, cons
 }
 
 // ------------------------------------------------------------------------------------------------
-// Cluster kernel for tableaus beyond one SM: one LP per thread-block cluster of C CTAs (C = 2, 4, 8, 16), the
-// tableau spread over the cluster's distributed shared memory.  Same algorithm, tolerances and pivot limit as
-// simplex_batch_kernel.
+// Dense-tableau kernel for every shape the warp kernel does not take: one LP per C CTAs (C = 1, 2, 4, 8, 16).  With
+// C = 1 one CTA holds the whole tableau in its shared memory; with C >= 2 the C CTAs form a thread-block cluster and
+// the tableau is spread over its distributed shared memory.
 //   column slices   CTA k owns the columns [k w, (k+1) w) of [A | I] for all m rows, and their lo, hi, cost, xn,
 //                   state and pivot-row entries;
 //   replicated rows every CTA keeps beta, basis, cb, colq and the bounds and cost of each row's basic variable;
-//   per pivot       pricing over the own columns + a cluster argmax of (value, index) (exchange 1: each CTA
+//   per pivot       pricing over the own columns + an argmax of (value, index) over the CTAs (exchange 1: each CTA
 //                   stores its candidate into every peer), then the owner of the entering column q stores colq and
 //                   q's scalars into every peer (exchange 2); the ratio test runs redundantly on the replicated rows
 //                   (same result everywhere, no exchange), the pivot row and the rank-1 update are local.
-// Two cluster barriers per pivot, no global memory inside the loop.  Determinism: every column's reduced cost,
-// pivot-row entry and update is the CTA kernel's expression with the same sequential loop over i; the argmax /
-// argmin order (value, then smallest index) is total, so the cluster reduction picks the CTA kernel's q and r.
-// Status, pivots, basis, x and y are therefore the CTA kernel's bytes; the objective's final sum is ordered
-// differently (one partial per CTA).  beta = b - A xN is formed by every CTA from global memory with the CTA
-// kernel's loop over j, so the replicated rows start identical in every CTA.
+// Two barriers over the LP's CTAs per pivot, no global memory inside the loop.  With C = 1 those are block barriers
+// and the exchanges are stores into the CTA's own shared memory: the kernel is launched without a cluster, so it pays
+// neither the cluster barrier nor its MEMBAR.ALL.GPU.
+// Determinism: every column's reduced cost, pivot-row entry and update is the same expression with the same
+// sequential loop over i as oracle/simplex_ref.c; the argmax / argmin order (value, then smallest index) is total, so
+// every C picks the same q and r.  Status, pivots, basis, x and y are therefore the same bytes for every C; the
+// objective is one block sum per CTA, added in rank order, so it matches across C only to the last bits.
 // ------------------------------------------------------------------------------------------------
 constexpr int SC_THREADS = 256;
 constexpr int SC_MAX_CTAS = 16;
 constexpr size_t SC_SMEM_MAX = 227 * 1024;
 
-// Per-CTA shared memory of the cluster kernel.  w = ceil((m + n) / C) rounded up to even (16-byte rows for the
+// Per-CTA shared memory of simplex_kernel.  w = ceil((m + n) / C) rounded up to even (16-byte rows for the
 // bulk copies).  Bytes = 8 m w (tableau slice) + 44 w (lo hi cost xn rowr, state) + 52 m (beta blo bhi bcost cb
 // colq, basis; m rounded up to even / to 4) + 368 (reduction scratch, exchange slots, q's scalars, mbarrier).
-struct ClusterSimplexLayout {
+struct SimplexLayout {
     int m, n, N, C, w;
     size_t off_T, off_beta, off_blo, off_bhi, off_bcost, off_cb, off_colq, off_lo, off_hi, off_cost, off_xn, off_rowr,
         off_redv, off_slotv, off_objv, off_q, off_bar, off_basis, off_state, off_redi, off_sloti, off_qstate, total;
-    __host__ __device__ ClusterSimplexLayout(int m_, int n_, int C_) : m(m_), n(n_), N(m_ + n_), C(C_) {
+    __host__ __device__ SimplexLayout(int m_, int n_, int C_) : m(m_), n(n_), N(m_ + n_), C(C_) {
         w = (((N + C - 1) / C) + 1) & ~1;
         auto up2 = [](size_t v) { return (v + 1) & ~(size_t)1; };
         size_t o = 0;
@@ -818,17 +525,33 @@ __device__ __forceinline__ double start_value(const double* lb, const double* ub
     return isfinite(l) ? l : (isfinite(u) ? u : 0.0);
 }
 
-__global__ void __launch_bounds__(SC_THREADS)
-simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict__ Ag, const double* __restrict__ bg,
-                       const double* __restrict__ cg_, const double* __restrict__ lbg, const double* __restrict__ ubg,
-                       const int8_t* __restrict__ senseg, int maximize, int max_pivots, int shared_model,
-                       int32_t* __restrict__ status_out, double* __restrict__ obj_out, double* __restrict__ x_out,
-                       double* __restrict__ y_out, int32_t* __restrict__ pivots_out, int32_t* __restrict__ basis_out) {
+// Barrier and peer address over the CTAs that hold one LP.  C = 1 runs without a cluster: a block barrier and the
+// CTA's own shared memory.
+__device__ __forceinline__ void lp_sync(int C) {
+    if (C == 1) __syncthreads();
+    else cooperative_groups::this_cluster().sync();
+}
+template <typename V>
+__device__ __forceinline__ V* lp_peer(V* p, int k, int C) {
+    return C == 1 ? p : cooperative_groups::this_cluster().map_shared_rank(p, (unsigned)k);
+}
+
+// CTAs per SM the 64-thread instance is compiled for: 12 hold it to 80 registers a thread (64 K / 768, rounded down to
+// the allocation unit), so a batch of small tableaus (m + n <= 96, e.g. 33 x 10) keeps 12 LPs per SM instead of the 8
+// that the 122 registers chosen otherwise allow.  0 leaves the other instances to the compiler (the same cap on the
+// 128-thread instance was 4 % slower on 24 x 144 MILPs and 2 % faster at 90 x 120, so it is not applied).
+constexpr int simplex_min_ctas(int threads) { return threads == 64 ? 12 : 0; }
+
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS, simplex_min_ctas(THREADS))
+simplex_kernel(int64_t B, int m, int n, int C, const double* __restrict__ Ag, const double* __restrict__ bg,
+               const double* __restrict__ cg_, const double* __restrict__ lbg, const double* __restrict__ ubg,
+               const int8_t* __restrict__ senseg, int maximize, int max_pivots, int shared_model,
+               int32_t* __restrict__ status_out, double* __restrict__ obj_out, double* __restrict__ x_out,
+               double* __restrict__ y_out, int32_t* __restrict__ pivots_out, int32_t* __restrict__ basis_out) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    namespace cgr = cooperative_groups;
-    cgr::cluster_group cluster = cgr::this_cluster();
-    constexpr int T = SC_THREADS;
-    const ClusterSimplexLayout lay(m, n, C);
+    constexpr int T = THREADS;
+    const SimplexLayout lay(m, n, C);
     const int N = lay.N, w = lay.w;
     double* sd = reinterpret_cast<double*>(smem_raw);
     double* Tl = sd + lay.off_T;                 // [m][w]: my columns of [A | I]
@@ -854,7 +577,7 @@ simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict_
     int* slot_i = reinterpret_cast<int*>(smem_raw + lay.off_sloti);
     int* qstate = reinterpret_cast<int*>(smem_raw + lay.off_qstate);
     const int tid = threadIdx.x;
-    const int rank = (int)cluster.block_rank();
+    const int rank = C == 1 ? 0 : (int)cooperative_groups::this_cluster().block_rank();
     const int j0 = rank * w;                                   // global id of my first column
     const int ns = min(max(n - j0, 0), w);                     // structural columns in my slice
 
@@ -907,21 +630,27 @@ simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict_
         const double l = lb ? lb[j] : 0.0, u = ub ? ub[j] : INFINITY;
         if (l > u) bad = 1;
     }
+    if (tA) mbar_wait(bar, 0);
     bad = __syncthreads_or(bad);
-    // replicated rows; beta = b - A xN with the CTA kernel's loop over j, read from global memory
+    // replicated rows; beta = b - A xN with one sequential loop over j.  One CTA reads A and xN from its own tableau
+    // and columns; the CTAs of a cluster each read them from global memory, so the rows start identical in every CTA.
     for (int i = tid; i < m; i += T) {
         const int s = sense ? sense[i] : 0;
         blo[i] = (s == ELP_GE) ? -INFINITY : 0.0;
         bhi[i] = (s == ELP_LE) ? INFINITY : 0.0;
         bcost[i] = 0.0;
         basis[i] = n + i;
-        const double* Ai = A + (size_t)i * n;
         double r = b[i];
-        for (int j = 0; j < n; ++j) r -= Ai[j] * start_value(lb, ub, j);
+        if (C == 1) {
+            const double* Ti = Tl + (size_t)i * w;
+            for (int j = 0; j < n; ++j) r -= Ti[j] * xn[j];
+        } else {
+            const double* Ai = A + (size_t)i * n;
+            for (int j = 0; j < n; ++j) r -= Ai[j] * start_value(lb, ub, j);
+        }
         beta[i] = r;
     }
-    if (tA) mbar_wait(bar, 0);
-    cluster.sync();       // every CTA of the cluster is running and staged before any peer store
+    lp_sync(C);       // every CTA of the LP is running and staged before any peer store
 
     int status = ELP_STATUS_TIMEOUT, pivots = 0, degenerate_run = 0, bland = 0;
     int qfinal = -1;
@@ -959,10 +688,10 @@ simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict_
         }
         cand = block_argmax<T>(cand, red_v, red_i);
         if (tid < C) {
-            cluster.map_shared_rank(slot_v, tid)[rank] = cand.v;
-            cluster.map_shared_rank(slot_i, tid)[rank] = cand.i;
+            lp_peer(slot_v, tid, C)[rank] = cand.v;
+            lp_peer(slot_i, tid, C)[rank] = cand.i;
         }
-        cluster.sync();
+        lp_sync(C);
         cand = ValIdx{slot_v[0], slot_i[0]};
         for (int k = 1; k < C; ++k) cand = better(cand, ValIdx{slot_v[k], slot_i[k]});
         if (cand.i < 0) { status = phase1 ? ELP_STATUS_INFEASIBLE : ELP_STATUS_OPTIMAL; break; }
@@ -973,16 +702,16 @@ simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict_
         // ---- entering column: its owner stores colq and q's scalars into every CTA (exchange 2) ------------------
         if (rank == qo) {
             for (int k = 0; k < C; ++k) {
-                double* dst = cluster.map_shared_rank(colq, k);
+                double* dst = lp_peer(colq, k, C);
                 for (int i = tid; i < m; i += T) dst[i] = Tl[i * w + ql];
             }
             if (tid < C) {
-                double* dq = cluster.map_shared_rank(qv, tid);
+                double* dq = lp_peer(qv, tid, C);
                 dq[0] = lo[ql]; dq[1] = hi[ql]; dq[2] = xn[ql]; dq[3] = cost[ql];
-                cluster.map_shared_rank(qstate, tid)[0] = state[ql];
+                lp_peer(qstate, tid, C)[0] = state[ql];
             }
         }
-        cluster.sync();
+        lp_sync(C);
         const double q_lo = qv[0], q_hi = qv[1], q_xn = qv[2], q_cost = qv[3];
         const int q_state = qstate[0];
         // ---- ratio test, pass 1 (replicated) ----------------------------------------------------------------------
@@ -1094,12 +823,12 @@ simplex_cluster_kernel(int64_t B, int m, int n, int C, const double* __restrict_
     }
     if (rank == 0) for (int i = tid; i < m; i += T) if (basis[i] < n) opart += bcost[i] * beta[i];
     const double part = block_sum<T>(opart, red_v);
-    if (tid == 0) cluster.map_shared_rank(obj_v, 0)[rank] = part;
-    cluster.sync();
+    if (tid == 0) lp_peer(obj_v, 0, C)[rank] = part;
+    lp_sync(C);
     if (rank == 0) {
         if (tid == 0) {
-            double obj = 0.0;
-            for (int k = 0; k < C; ++k) obj += obj_v[k];
+            double obj = obj_v[0];      // C = 1: the block sum itself, a -0.0 included
+            for (int k = 1; k < C; ++k) obj += obj_v[k];
             if (status == ELP_STATUS_UNBOUNDED) obj = -INFINITY;
             status_out[lp] = status;
             obj_out[lp] = maximize ? -obj : obj;
@@ -1127,22 +856,20 @@ __global__ void k_densify(int m, int n, const int* __restrict__ ptr, const int* 
     for (int k = ptr[i] + threadIdx.x; k < ptr[i + 1]; k += blockDim.x) atomicAdd(&A[(size_t)i * n + idx[k]], val[k]);
 }
 
-size_t simplex_smem_bytes(int m, int n) { return SimplexSmemLayout(m, n).total; }
+// ELP_METHOD_AUTO's size rule: simplex when the dense tableau fits 200 KB.
+// Stated on the former one-SM kernel's footprint, so that AUTO picks the same method for every shape as before.
+bool simplex_auto_prefers(int m, int n) {
+    auto up2 = [](size_t v) { return (v + 1) & ~(size_t)1; };
+    auto up4 = [](size_t v) { return (v + 3) & ~(size_t)3; };
+    const size_t N = (size_t)m + n;
+    const size_t bytes = 8 * (up2((size_t)m * n) + up2((size_t)m * m) + 3 * up2(m) + 5 * up2(N) + 8) + 16 +
+                         4 * (up4(m) + up4(N) + 8);
+    return bytes <= 200 * 1024;
+}
 
 static int env_flag(const char* name, int dflt) {
     const char* e = getenv(name);
     return e ? atoi(e) : dflt;
-}
-
-int simplex_pick_threads(int m, int n) {
-    const int N = m + n;
-    if (const char* e = getenv("ELP_SIMPLEX_THREADS")) {
-        const int t = atoi(e);
-        if (t == 32 || t == 64 || t == 128) return t;
-    }
-    if (N <= 32) return 32;
-    if (N <= 96) return 64;
-    return 128;
 }
 
 // Warp-per-LP path: returns false when the shape does not fit the register tableau (caller falls back).
@@ -1192,8 +919,9 @@ static bool simplex_warp_launch(int64_t B, int m, int n, const double* A, const 
 // Can the device schedule one cluster of C CTAs with this much shared memory each?  C = 16 is a non-portable size.
 static bool cluster_schedulable(int C, size_t smem) {
     if (smem > SC_SMEM_MAX) return false;
-    ELP_CUDA(cudaFuncSetAttribute(simplex_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (C > 8) ELP_CUDA(cudaFuncSetAttribute(simplex_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    const auto kern = simplex_kernel<SC_THREADS>;
+    ELP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (C > 8) ELP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)C);
     cfg.blockDim = dim3(SC_THREADS);
@@ -1203,35 +931,35 @@ static bool cluster_schedulable(int C, size_t smem) {
     at[0].val.clusterDim.x = (unsigned)C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
     int clusters = 0;
-    if (cudaOccupancyMaxActiveClusters(&clusters, simplex_cluster_kernel, &cfg) != cudaSuccess) {
+    if (cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg) != cudaSuccess) {
         cudaGetLastError();
         return false;
     }
     return clusters >= 1;
 }
 
-// The one place that decides how many CTAs hold one LP's tableau: 1 (the warp kernel, else the CTA kernel: one SM)
-// or C (the cluster kernel, the smallest C in {2, 4, 8, 16} that fits and can be scheduled).  ELP_SIMPLEX_CLUSTER=C
-// forces the cluster kernel with C CTAs on any shape it can hold.  Throws when no kernel can take the shape.
+// The one place that decides how many CTAs hold one LP's tableau: 1 (the warp kernel, else one CTA of simplex_kernel:
+// one SM) or C (a cluster of simplex_kernel, the smallest C in {2, 4, 8, 16} that fits and can be scheduled).
+// ELP_SIMPLEX_CLUSTER=C forces a cluster of C CTAs on any shape it can hold.  Throws when no kernel can take the shape.
 int simplex_ctas(int m, int n) {
     const char* e = getenv("ELP_SIMPLEX_CLUSTER");
     const int forced = e ? atoi(e) : 0;
     if (forced == 2 || forced == 4 || forced == 8 || forced == 16) {
-        if (cluster_schedulable(forced, ClusterSimplexLayout(m, n, forced).total)) return forced;
+        if (cluster_schedulable(forced, SimplexLayout(m, n, forced).total)) return forced;
     }
-    if (simplex_smem_bytes(m, n) <= SC_SMEM_MAX) return 1;
+    if (SimplexLayout(m, n, 1).total <= SC_SMEM_MAX) return 1;
     int largest = 0;
     for (int C = 2; C <= SC_MAX_CTAS; C *= 2) {
-        if (!cluster_schedulable(C, std::min(ClusterSimplexLayout(m, n, C).total, SC_SMEM_MAX))) continue;
+        if (!cluster_schedulable(C, std::min(SimplexLayout(m, n, C).total, SC_SMEM_MAX))) continue;
         largest = C;
-        if (ClusterSimplexLayout(m, n, C).total <= SC_SMEM_MAX) return C;
+        if (SimplexLayout(m, n, C).total <= SC_SMEM_MAX) return C;
     }
     int ncap = 0;          // structural columns the largest schedulable cluster holds at this row count
     if (largest) {
         int lo = 0, hi = 1 << 24;
         while (lo < hi) {
             const int mid = lo + (hi - lo + 1) / 2;
-            if (ClusterSimplexLayout(m, mid, largest).total <= SC_SMEM_MAX) lo = mid;
+            if (SimplexLayout(m, mid, largest).total <= SC_SMEM_MAX) lo = mid;
             else hi = mid - 1;
         }
         ncap = lo;
@@ -1250,8 +978,8 @@ int simplex_batch_device(int64_t B, int m, int n, const double* A, const double*
     const int ctas = simplex_ctas(m, n);
     if (B <= 0) return ctas;
     ELP_REQUIRE(B * ctas < 0x7fffffffll, "simplex: batch too large");
+    const size_t smem = SimplexLayout(m, n, ctas).total;
     if (ctas > 1) {
-        const size_t smem = ClusterSimplexLayout(m, n, ctas).total;
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)(B * ctas));
         cfg.blockDim = dim3(SC_THREADS);
@@ -1262,25 +990,18 @@ int simplex_batch_device(int64_t B, int m, int n, const double* A, const double*
         at[0].val.clusterDim.x = (unsigned)ctas; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
         g_launches.fetch_add(1, std::memory_order_relaxed);
-        ELP_CUDA(cudaLaunchKernelEx(&cfg, simplex_cluster_kernel, B, m, n, ctas, A, b, c, lb, ub, sense, maximize,
+        ELP_CUDA(cudaLaunchKernelEx(&cfg, simplex_kernel<SC_THREADS>, B, m, n, ctas, A, b, c, lb, ub, sense, maximize,
                                     max_pivots, shared_model, status, obj, x, y, pivots, basis));
         ELP_CUDA(cudaGetLastError());
         return ctas;
     }
     if (simplex_warp_launch(B, m, n, A, b, c, lb, ub, sense, maximize, max_pivots, status, obj, x, y, pivots, st, shared_model, basis)) return 1;
-    const size_t smem = simplex_smem_bytes(m, n);
-    const int threads = simplex_pick_threads(m, n);
-#define ELP_SIMPLEX_LAUNCH(T)                                                                                     \
-    do {                                                                                                          \
-        ELP_CUDA(cudaFuncSetAttribute(simplex_batch_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
-                                      (int)smem));                                                                \
-        ELP_LAUNCH((simplex_batch_kernel<T>), (unsigned)B, T, smem, st, B, m, n, A, b, c, lb, ub, sense, maximize, \
-                   max_pivots, shared_model, status, obj, x, y, pivots, basis);                                   \
-    } while (0)
-    if (threads == 32) ELP_SIMPLEX_LAUNCH(32);
-    else if (threads == 64) ELP_SIMPLEX_LAUNCH(64);
-    else ELP_SIMPLEX_LAUNCH(128);
-#undef ELP_SIMPLEX_LAUNCH
+    // one CTA per LP, launched without a cluster: 32, 64 or 128 threads by the width m + n
+    const int N = m + n, threads = N <= 32 ? 32 : (N <= 96 ? 64 : 128);
+    const auto kern = threads == 32 ? simplex_kernel<32> : (threads == 64 ? simplex_kernel<64> : simplex_kernel<128>);
+    ELP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ELP_LAUNCH(kern, (unsigned)B, threads, smem, st, B, m, n, 1, A, b, c, lb, ub, sense, maximize, max_pivots, shared_model,
+               status, obj, x, y, pivots, basis);
     return 1;
 }
 

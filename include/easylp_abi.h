@@ -94,7 +94,7 @@ typedef struct elp_stats {
     double spmv_ms;            /* device time of the timed A.x / A'.y probe (elp_pdlp_probe_spmv) */
     int32_t limit_reached;     /* with status 7: 0 = only this call's max_new_iters ran out (call again), 1 = the iteration
                                   limit of the solve, 2 = its time limit (lp.control(timeout=)) — do not call again */
-    int32_t simplex_ctas;      /* CTAs that held each simplex tableau: 0 PDLP ran, 1 one SM (warp or CTA kernel), C a
+    int32_t simplex_ctas;      /* CTAs that held each simplex tableau: 0 PDLP ran, 1 one SM (a warp or one CTA), C a
                                   thread-block cluster of C CTAs (tableaus beyond one SM's shared memory) */
 } elp_stats;
 

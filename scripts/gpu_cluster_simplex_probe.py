@@ -1,6 +1,6 @@
 """Simplex on a thread-block cluster: per-pivot cost of the cluster kernel on medium LPs, against PDLP to 1e-6 on the same
 LP, HiGHS' dual simplex on one CPU core (a stand-in for lp_solve, which is not available here) and branch and bound on
-MILPs beyond one SM; the forced cluster kernel against the one-SM CTA kernel on a shape both take.
+MILPs beyond one SM; forced clusters against the one-CTA instance on a shape one SM holds.
 
     python scripts/gpu_cluster_simplex_probe.py [out.json]
 
@@ -100,7 +100,7 @@ def main():
                    nodes_per_s=r.stats.restarts / (wall / 1e3))
         res["mip"].append(row)
         print(json.dumps(row), flush=True)
-    # forced cluster against the CTA kernel on shapes both take
+    # forced clusters against the one-CTA instance on shapes one SM holds
     for (m, n) in [(90, 120), (60, 150)]:
         p = T.mixed(m, n, 5)
         p["maximize"] = False

@@ -1,6 +1,6 @@
-"""Simplex on a thread-block cluster (csrc/simplex.cu, simplex_cluster_kernel): LPs, MILPs and sensitivity ranging whose
-dense tableau [A | I] does not fit one SM's shared memory.  CPU: the C oracle agrees with HiGHS on every family used
-below.  GPU: the cluster kernel forced onto shapes the CTA kernel takes gives the CTA kernel's bytes (status, pivots,
+"""Simplex on a thread-block cluster (csrc/simplex.cu, simplex_kernel with C >= 2 CTAs): LPs, MILPs and sensitivity
+ranging whose dense tableau [A | I] does not fit one SM's shared memory.  CPU: the C oracle agrees with HiGHS on every
+family used below.  GPU: clusters forced onto shapes one CTA holds give the one-CTA instance's bytes (status, pivots,
 basis-derived x and y, ranging); beyond one SM it agrees with the oracle and HiGHS; shapes beyond the largest cluster
 are refused with an error naming the shape and the capacity; the AUTO size rule is unchanged."""
 import numpy as np
@@ -16,22 +16,22 @@ def _up2(v):
     return (v + 1) & ~1
 
 
-def cta_bytes(m, n):
-    """shared memory of the one-SM CTA kernel (SimplexSmemLayout)"""
+def auto_bytes(m, n):
+    """ELP_METHOD_AUTO's footprint (simplex_auto_prefers: simplex when it is at most 200 KB)"""
     N = m + n
     d = _up2(m * n) + _up2(m * m) + _up2(m) + 4 * _up2(N) + _up2(m) + _up2(m) + _up2(N) + 8
     return d * 8 + 16 + ((m + 3) & ~3) * 4 + ((N + 3) & ~3) * 4 + 32
 
 
 def cluster_bytes(m, n, C):
-    """per-CTA shared memory of the cluster kernel (ClusterSimplexLayout)"""
+    """per-CTA shared memory of simplex_kernel with C CTAs per LP (SimplexLayout)"""
     w = (((m + n + C - 1) // C) + 1) & ~1
     d = m * w + 6 * _up2(m) + 5 * w + 8 + 16 + 16 + 4
     return d * 8 + 16 + ((m + 3) & ~3) * 4 + ((w + 3) & ~3) * 4 + 32 + 64 + 16
 
 
 def expected_ctas(m, n, largest):
-    if cta_bytes(m, n) <= SMEM_MAX:
+    if cluster_bytes(m, n, 1) <= SMEM_MAX:
         return 1
     for C in (2, 4, 8, 16):
         if C <= largest and cluster_bytes(m, n, C) <= SMEM_MAX:
@@ -162,7 +162,7 @@ def random_ranging_lp(seed, m=120, n=300):
                 c=rng.uniform(0.5, 4.0, size=n), lb=np.zeros(n), ub=np.full(n, 20.0), maximize=True, A=A)
 
 
-BEYOND = [("transport", 60, 800), ("planted", 80, 300), ("planted", 200, 700), ("planted", 250, 700)]
+BEYOND = [("transport", 60, 800), ("planted", 80, 300), ("planted", 200, 700), ("planted", 250, 700), ("planted", 100, 170)]
 
 
 # ---- CPU: the oracle is sound at these sizes ---------------------------------------------------------------------------
@@ -194,6 +194,7 @@ def test_size_rule_places_the_issue_shapes():
     assert expected_ctas(60, 800, 16) == 2 and expected_ctas(80, 300, 16) == 2 and expected_ctas(50, 625, 16) == 2
     assert expected_ctas(200, 700, 16) == 8
     assert expected_ctas(250, 700, 16) == 16 and expected_ctas(250, 700, 8) is None
+    assert expected_ctas(100, 150, 16) == 1 and expected_ctas(100, 170, 16) == 2
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------------------
@@ -234,7 +235,7 @@ def _same_bits(a, b):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("m,n", [(40, 100), (60, 150), (90, 120)])
-def test_forced_cluster_gives_the_cta_kernels_bytes_through_solve_lp(m, n, monkeypatch, largest_cluster):
+def test_forced_cluster_gives_the_one_cta_instances_bytes_through_solve_lp(m, n, monkeypatch, largest_cluster):
     statuses = set()
     for seed in range(12):
         p = mixed(m, n, 1000 * m + seed)
@@ -255,7 +256,7 @@ def test_forced_cluster_gives_the_cta_kernels_bytes_through_solve_lp(m, n, monke
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("m,n", [(40, 100), (90, 120)])
-def test_forced_cluster_gives_the_cta_kernels_bytes_through_solve_batch(m, n, monkeypatch, largest_cluster):
+def test_forced_cluster_gives_the_one_cta_instances_bytes_through_solve_batch(m, n, monkeypatch, largest_cluster):
     ps = [mixed(m, n, 7 * m + s) for s in range(24)]
     A = np.stack([p["A"] for p in ps]); b = np.stack([p["rhs"] for p in ps]); c = np.stack([p["c"] for p in ps])
     lb = np.stack([p["lb"] for p in ps]); ub = np.stack([p["ub"] for p in ps]); sense = np.stack([p["sense"] for p in ps])
@@ -274,7 +275,7 @@ def test_forced_cluster_gives_the_cta_kernels_bytes_through_solve_batch(m, n, mo
 
 
 @pytest.mark.gpu
-def test_forced_cluster_gives_the_cta_kernels_ranging(monkeypatch, largest_cluster):
+def test_forced_cluster_gives_the_one_cta_instances_ranging(monkeypatch, largest_cluster):
     checked = 0
     for seed in range(6):
         p = random_ranging_lp(seed, m=40, n=100)
@@ -442,3 +443,9 @@ def test_auto_keeps_its_size_rule(monkeypatch):
     small = planted(40, 100, 3)
     r = _solve(small, monkeypatch, method=L.METHOD_AUTO)
     assert r.stats.method_used == L.METHOD_SIMPLEX and r.stats.simplex_ctas == 1
+    # the rule stays on its own footprint: 100 x 135 is below 200 KB there (not on the one-CTA footprint), 100 x 140 above
+    assert auto_bytes(100, 135) <= 200 * 1024 < cluster_bytes(100, 135, 1) and auto_bytes(100, 140) > 200 * 1024
+    r = _solve(planted(100, 135, 3), monkeypatch, method=L.METHOD_AUTO)
+    assert r.stats.method_used == L.METHOD_SIMPLEX and r.stats.simplex_ctas == 1
+    r = _solve(planted(100, 140, 3), monkeypatch, method=L.METHOD_AUTO)
+    assert r.stats.method_used == L.METHOD_PDLP

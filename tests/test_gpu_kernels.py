@@ -330,7 +330,7 @@ def test_pdlp_transport_vs_simplex_oracle():
                                  (28, 30), (32, 60), (5, 70), (10, 86), (33, 10), (20, 80), (40, 100)])
 def test_batch_shapes_vs_oracle(m, n):
     """every register-tableau instantiation (rows padded to 4, 1-3 columns per lane), odd sizes (no TMA path) and
-    the shapes that fall back to the CTA-per-LP kernel"""
+    the shapes that run one LP per CTA"""
     rng = np.random.default_rng(100 * m + n)
     B = 300
     A = rng.uniform(-0.3, 1.0, size=(B, m, n)) * (rng.random((B, m, n)) < 0.8)
